@@ -7,7 +7,7 @@ with ess_perc_min = 1.0, so the stratified resample + gather of all six planes r
 setting of the reference's own benchmark, benchmarks/ssm/WeightedSampling/lgssm1d.jl:26-27).
 particle-updates/s = N * steps / time.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--particles N] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--particles N] [--impl reference] [--dump-outputs DIR]
 
 * `value`     device time of the K steps (CUDA events on the library's stream), library timing hooks OFF.
 * `e2e`       the same K steps through the public API (wsb200.run of the @model program) with host
@@ -23,6 +23,9 @@ particle-updates/s = N * steps / time.
 * `cpu_baseline` / `--impl reference`  the C restatement of the reference's run! (oracle/ws_oracle.c:
               orc_ssm2d_run) on one host core (the reference is single-threaded: TODO.md:28).  Julia is
               not available, so this is "kind: port".
+* `--dump-outputs DIR`  after the timed steps, writes what they computed as DIR/<name>.npy (float64): the particle
+              columns x, v, dv and the log-weights at a fixed, seeded sample of particles, and the log-evidence.  The
+              inputs depend only on the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -204,6 +207,28 @@ def sharded_parity(ws, dist, torch, local_rank, rank, world, n=200_003, T=12):
     return out
 
 
+DUMP_PARTICLES = 1_000_000      # 7 float64 values per sampled particle: 56 MB in all, whatever --particles is
+
+
+def dump_outputs(state, le, out_dir, rank, world):
+    """Writes the state a caller of ws.run holds after the timed steps.  The sample of particles is seeded, so it
+    depends only on the particle count; rows are read through the deferred ancestors, which leaves the state as it was."""
+    import ctypes as C
+    st = state.store
+    m = min(st.n, DUMP_PARTICLES // world)
+    rows = np.sort(np.random.default_rng(0).choice(st.n, size=m, replace=False)).astype(np.int64)
+    out = {"log_evidence": np.array([le]), "log_weights": state.weights[rows]}
+    for name in ("x", "v", "dv"):
+        cid, width = st._lookup(name)
+        planes = np.empty((width, m))
+        st._call("ws_col_download_rows", cid, rows.ctypes.data_as(C.c_void_p), m, planes.ctypes.data_as(C.c_void_p))
+        out[name] = np.ascontiguousarray(planes.T)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f"_rank{rank}"
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a)
+
+
 def cpu_reference_run(n, steps, seed=1):
     """The reference's run! restated in C (oracle/ws_oracle.c), one core."""
     from oracle import cref
@@ -257,7 +282,12 @@ def main():
     ap.add_argument("--profile-steps", type=int, default=10, help="steps of the second pass that times each kernel class")
     ap.add_argument("--skew", type=float, default=2.0, help="N > 1: rank skew of the extra migration-heavy Resample (0 = skip it)")
     ap.add_argument("--eager-gather", action="store_true", help="gather every column inside Resample (reference order of work)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed steps computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -357,6 +387,8 @@ def main():
     chunk_ms_per_step = [evs[i].elapsed_time(evs[i + 1]) / (cuts[i + 1] - cuts[i]) for i in range(n_chunks)]
     clocks = sampler.stop()
     stats1 = state.stats()
+    if args.dump_outputs:
+        dump_outputs(state, le, args.dump_outputs, rank, world)
     # second pass, NOT part of the headline: the same filter continues for KP steps with per-kernel events on
     st._call("ws_set_timing", 1)
     st._call("ws_reset_kernel_times")
