@@ -951,6 +951,9 @@ __device__ __forceinline__ int64_t ws_F(const WsScanParams& P, double C, double 
 //                     no loop per particle; the test-suite checks it against exact big-integer arithmetic.
 #define WS_TILE_GROUP 32       // CDF tiles per group of the two-level tile offsets
 #define WS_EXPAND_CHUNK 512    // output slots a warp stages in shared memory per round
+#ifndef WS_EXPAND_LANE
+#define WS_EXPAND_LANE 12      // staged slots a lane resolves per round of the running maximum (a multiple of 4)
+#endif
 #define WS_DIRECT_MAX 8        // offspring a lane writes itself; larger families are filled by the warp
 #define WS_WARPS_PER_CTA (WS_SCAN_BLOCK / 32)
 #define WS_MN_MAX_WINDOWS 64   // multinomial: windows of WS_RBUF_SLOTS slots a warp works through before the tile counts as heavy
@@ -990,14 +993,15 @@ __device__ __forceinline__ int ws_F_int(unsigned long long C, unsigned int n, in
 #define WS_CDF_ASYNC 0   // (measured, profiles/r2o_scan_variants.txt: registers 0.74 ms, cp.async 0.81 ms for scan + search at N = 1e8) next tile's log-weights by cp.async into shared memory (1) or by plain loads into registers (0)
 #endif
 #ifndef WS_CDF_MINB
-#define WS_CDF_MINB 5   // <= 51 registers: five CTAs per SM (measured against 1 / 4 with grids of 3, 4, 8 CTAs per SM)
+#define WS_CDF_MINB 4   // <= 64 registers, four CTAs per SM: no spills (at five CTAs, 48 registers, the prefetched tile spilled)
 #endif
 #ifndef WS_CDF_GRID
-#define WS_CDF_GRID 5
+#define WS_CDF_GRID 4
 #endif
 __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_CDF_MINB) ws_cdf_tiles_kernel(const __grid_constant__ WsScanParams P) {
     if (P.gate != 0 && P.red->do_resample == 0) return;
-    __shared__ unsigned long long warp_tot[WS_SCAN_BLOCK / 32];
+    __shared__ unsigned long long warp_tot[2][WS_SCAN_BLOCK / 32];
+    int parity = 0;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int n = (int)P.n;
     const int n_tiles = (n + WS_CDF_TILE - 1) / WS_CDF_TILE;
@@ -1049,7 +1053,7 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_CDF_MINB) ws_cdf_tiles_kerne
                 // saturating conversion (NaN -> 0) is ws_w_to_fxs without its two compares
 #pragma unroll
                 for (int k = 0; k < WS_SCAN_ITEMS; ++k)
-                    q[k] = __double2ull_rn(ws_div_pos(ws_exp_nonpos(l[k] - m), Sden, rS) * P.fx_scale);
+                    q[k] = __double2ull_rn(ws_div_pos(ws_exp_nonpos_or0(l[k] - m), Sden, rS) * P.fx_scale);
             } else {
 #pragma unroll
                 for (int k = 0; k < WS_SCAN_ITEMS; ++k) q[k] = (item0 + k < n) ? ws_w_to_fxs(l[k], P.fx_scale) : 0ull;
@@ -1073,10 +1077,13 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_CDF_MINB) ws_cdf_tiles_kerne
             for (int k = 0; k < WS_SCAN_ITEMS; ++k) l[k] = (item0 + k < n) ? __ldg(P.logw + item0 + k) : -INFINITY;
         }
     };
-    double l_next[WS_SCAN_ITEMS];
+    // A landed tile is converted to fixed point before the next one is requested, so that only one set of eight
+    // 64-bit values (the loads in flight, then q) is live besides the other: holding l, l_next and q together spilled
+    // under the five-CTA register cap.
+    double l[WS_SCAN_ITEMS];
 #pragma unroll
-    for (int k = 0; k < WS_SCAN_ITEMS; ++k) l_next[k] = -INFINITY;
-    if (P.mode != 2 && (int)blockIdx.x < n_tiles) load_tile(blockIdx.x, l_next);
+    for (int k = 0; k < WS_SCAN_ITEMS; ++k) l[k] = -INFINITY;
+    if (P.mode != 2 && (int)blockIdx.x < n_tiles) load_tile(blockIdx.x, l);
     for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const int item0 = tile * WS_CDF_TILE + threadIdx.x * WS_SCAN_ITEMS;
         unsigned long long q[WS_SCAN_ITEMS];
@@ -1084,20 +1091,17 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_CDF_MINB) ws_cdf_tiles_kerne
 #pragma unroll
             for (int k = 0; k < WS_SCAN_ITEMS; ++k) q[k] = (item0 + k < n) ? ws_w_to_fxs(uniform_w, P.fx_scale) : 0ull;
         } else {
-            double l[WS_SCAN_ITEMS];
-#pragma unroll
-            for (int k = 0; k < WS_SCAN_ITEMS; ++k) l[k] = l_next[k];
-            if (tile + (int)gridDim.x < n_tiles) load_tile(tile + gridDim.x, l_next);
             if (P.mode == 0) {
-                // items beyond the shard were loaded as -inf: e = 0.  e <= 1 and S >= 1, so w is in [0, 1] or NaN and the
-                // saturating conversion (NaN -> 0) is ws_w_to_fxs without its two compares
+                // items beyond the shard were loaded as -inf: e = 0.  e <= 1 and S >= 1, so w is in [0, 1] and the
+                // conversion is ws_w_to_fxs without its two compares; NaN, -inf and d < -708 all give e = 0, q = 0
 #pragma unroll
                 for (int k = 0; k < WS_SCAN_ITEMS; ++k)
-                    q[k] = __double2ull_rn(ws_div_pos(ws_exp_nonpos(l[k] - m), Sden, rS) * P.fx_scale);
+                    q[k] = __double2ull_rn(ws_div_pos(ws_exp_nonpos_or0(l[k] - m), Sden, rS) * P.fx_scale);
             } else {
 #pragma unroll
                 for (int k = 0; k < WS_SCAN_ITEMS; ++k) q[k] = (item0 + k < n) ? ws_w_to_fxs(l[k], P.fx_scale) : 0ull;
             }
+            if (tile + (int)gridDim.x < n_tiles) load_tile(tile + gridDim.x, l);
         }
 #endif
 #pragma unroll
@@ -1109,16 +1113,22 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_CDF_MINB) ws_cdf_tiles_kerne
             unsigned long long t = __shfl_up_sync(0xffffffffu, incl, d);
             if (lane >= d) incl += t;
         }
-        __syncthreads();  // warp_tot of the previous tile has been consumed
-        if (lane == 31) warp_tot[warp] = incl;
+        // two sets of warp totals, alternating with the tile: a warp writes set p only after the barrier of the tile in
+        // between, which every warp passes after it has read set p, so one barrier per tile suffices
+        unsigned long long* const wt = warp_tot[parity];
+        parity ^= 1;
+        if (lane == 31) wt[warp] = incl;
         __syncthreads();
-        unsigned long long warp_excl = 0ull, tile_agg = 0ull;
+        // lanes 0..7 take one warp total each: a shuffle scan over them gives the warp's exclusive prefix and the tile's sum
+        unsigned long long t8 = lane < WS_SCAN_BLOCK / 32 ? wt[lane] : 0ull;
 #pragma unroll
-        for (int w = 0; w < WS_SCAN_BLOCK / 32; ++w) {
-            const unsigned long long t = warp_tot[w];
-            if (w < warp) warp_excl += t;
-            tile_agg += t;
+        for (int d = 1; d < WS_SCAN_BLOCK / 32; d <<= 1) {
+            const unsigned long long t = __shfl_up_sync(0xffffffffu, t8, d);
+            if (lane >= d) t8 += t;
         }
+        const unsigned long long tile_agg = __shfl_sync(0xffffffffu, t8, WS_SCAN_BLOCK / 32 - 1);
+        unsigned long long warp_excl = __shfl_sync(0xffffffffu, t8, (warp + 31) & 31);
+        if (warp == 0) warp_excl = 0ull;
         const unsigned long long thread_excl = warp_excl + (incl - thread_total);
         if (item0 + WS_SCAN_ITEMS <= n) {
             ulonglong2* dst = reinterpret_cast<ulonglong2*>(P.cdf_local + item0);
@@ -1404,15 +1414,24 @@ __device__ __forceinline__ void ws_search_setup(const WsScanParams& P, WsSearchC
 #ifndef WS_INTERIOR_FAST
 #define WS_INTERIOR_FAST 1   // 0: every tile takes the range-checked search (A/B)
 #endif
+#define WS_RING_BLOCKS 128u   // Philox blocks (16 B each) a warp keeps from one tile to the next (power of two)
+// A warp's Philox blocks carried from tile to tile (Philox-stratified interior tiles): blocks [lo, hi) are valid, block
+// b is buf[b % WS_RING_BLOCKS], its words masked with rmask.  Every lane holds the same lo and hi.
+struct WsRing {
+    uint4* buf;
+    unsigned int lo, hi;
+};
 // One warp, one tile of WS_SCAN_TILE consecutive particles starting at `tile_base`, lane L holding the global
 // fixed-point CDF C[k] of particles tile_base + 8 L + k: per-particle slot counts F(C_m), then the offspring slots
 // [F(C_{m-1}), F(C_m)) of every particle are written to P.ancestors.  `Cp` (lane 0; valid iff has_prev) is the CDF of
-// the particle in front of the tile.  `rbuf`: the warp's shared-memory window (WS_RBUF_SLOTS words).
-template <bool EXACT_FP, bool MN>
+// the particle in front of the tile.  `rbuf`: the warp's shared-memory window (WS_RBUF_SLOTS words).  SHR: the slot
+// split's shift X.sh is known to be >= 0 (N <= 2^29 without WSB200_FX_EXTRA_BITS).  `ring` (optional): the warp's
+// Philox ring, for a warp that searches consecutive tiles.
+template <bool EXACT_FP, bool MN, bool SHR = false>
 __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSearchCtx& X, unsigned long long* const rbuf,
                                                     const int lane, const int tile_base,
                                                     const unsigned long long (&C)[WS_SCAN_ITEMS], const unsigned long long Cp,
-                                                    const bool has_prev, const bool interior = false) {
+                                                    const bool has_prev, const bool interior = false, WsRing* const ring = nullptr) {
     int32_t* const out_s = reinterpret_cast<int32_t*>(rbuf);
     unsigned int* const rbuf32 = reinterpret_cast<unsigned int*>(rbuf);
     SlotUniform& su = X.su;
@@ -1425,7 +1444,7 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
     // particle 1, as in icdf); elsewhere it is the previous particle's F.
     int f[WS_SCAN_ITEMS];
     int fstart = slot_base;
-    bool coop = false;
+    bool coop = false, ringed = false;
     if (!EXACT_FP && MN) {
         // Multinomial: thresholds T_m of the lane's particles in the units of the spacing sums; the warp finds the
         // blocks of slots the tile can reach, regenerates their spacings once (running sums in the shared window)
@@ -1534,7 +1553,7 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
         const unsigned int last = (unsigned int)ns - 1u;
 #pragma unroll
         for (int k = 0; k < WS_SCAN_ITEMS; ++k) {
-            const unsigned long long T = sh >= 0 ? (C[k] >> sh) : (C[k] << (-sh));
+            const unsigned long long T = (SHR || sh >= 0) ? (C[k] >> sh) : (C[k] << (-sh));
             kk[k] = (unsigned int)(T >> 32);
             fr[k] = (unsigned int)T;
             if (kk[k] > last) {
@@ -1544,7 +1563,7 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
         }
         unsigned int kp = kk[0], frp = 0u;
         if (lane == 0 && has_prev) {
-            const unsigned long long T = sh >= 0 ? (Cp >> sh) : (Cp << (-sh));
+            const unsigned long long T = (SHR || sh >= 0) ? (Cp >> sh) : (Cp << (-sh));
             kp = (unsigned int)(T >> 32);
             frp = (unsigned int)T;
             if (kp > last) {
@@ -1553,9 +1572,29 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
             }
         }
         const unsigned int blk0 = __shfl_sync(0xffffffffu, kp, 0) >> 2;
-        const unsigned int nblk = (__shfl_sync(0xffffffffu, kk[WS_SCAN_ITEMS - 1], 31) >> 2) - blk0 + 1u;
+        const unsigned int blk1 = __shfl_sync(0xffffffffu, kk[WS_SCAN_ITEMS - 1], 31) >> 2;
+        const unsigned int nblk = blk1 - blk0 + 1u;
         coop = nblk <= (unsigned int)(WS_RBUF_SLOTS / 2);
-        if (coop) {
+        if (ring != nullptr && nblk <= WS_RING_BLOCKS - 32u) {
+            // The ring keeps the blocks a warp generated for its previous tiles: consecutive tiles share their boundary
+            // block, and a round of 32 blocks that overshoots the tile serves the next one.  A round writes blocks
+            // [hi, hi + 32) over [hi - WS_RING_BLOCKS, ...), which lie below blk0 as long as nblk <= WS_RING_BLOCKS - 32.
+            if (blk0 < ring->lo || blk0 >= ring->hi) ring->lo = ring->hi = blk0;
+            __syncwarp();   // every lane is done reading the blocks this round replaces
+            for (; ring->hi <= blk1; ring->hi += 32u) {
+                const unsigned int b = ring->hi + (unsigned int)lane;
+                const ws_u32x4 r = ws_philox4x32_10((uint64_t)b, P.stream, P.seed);
+                ring->buf[b & (WS_RING_BLOCKS - 1u)] = make_uint4(r.x & rmask, r.y & rmask, r.z & rmask, r.w & rmask);
+            }
+            if (ring->hi - ring->lo > WS_RING_BLOCKS) ring->lo = ring->hi - WS_RING_BLOCKS;
+            __syncwarp();
+            const unsigned int* const rb = reinterpret_cast<const unsigned int*>(ring->buf);
+            constexpr unsigned int RMASK = 4u * WS_RING_BLOCKS - 1u;
+#pragma unroll
+            for (int k = 0; k < WS_SCAN_ITEMS; ++k) f[k] = (int)kk[k] + (rb[kk[k] & RMASK] <= fr[k] ? 1 : 0);
+            if (lane == 0 && has_prev) fstart = (int)kp + (rb[kp & RMASK] <= frp ? 1 : 0);
+            coop = ringed = true;
+        } else if (coop) {
             for (unsigned int b = lane; b < nblk; b += 32u) {
                 const ws_u32x4 r = ws_philox4x32_10((uint64_t)(blk0 + b), P.stream, P.seed);
                 reinterpret_cast<uint4*>(rbuf32)[b] = make_uint4(r.x & rmask, r.y & rmask, r.z & rmask, r.w & rmask);
@@ -1646,6 +1685,8 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
             else fstart = ws_F_int(Cp, (unsigned int)ns, sh, rmask, su.scheme, r0_int, P.seed, P.stream);
         }
     }
+    // the other paths use the whole window for their slot uniforms, the ring's half included
+    if (ring != nullptr && !ringed) ring->lo = ring->hi = 0u;
     // items beyond the shard produce nothing: they repeat the F of the shard's last particle
     if (!interior) {
         const int rank_end = P.bounds != nullptr ? P.bounds[1] : ns;
@@ -1675,52 +1716,61 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
     }
 
     // ---- expand: offspring slots [F(C_{m-1}), F(C_m)) of particle m ---------------------------------
-    if (fend - fstart <= WS_EXPAND_CHUNK) {
-        // the common case: the tile's slots fit one staging window.  Every particle with offspring marks
-        // the FIRST of its slots with its index + 1 (one predicated store, no divergence on the family
-        // size); the other slots take the last mark before them (a running maximum: marks increase with
-        // the slot), resolved four slots per lane and round and written as 16-byte stores.
+    constexpr int PL = WS_EXPAND_LANE, PR = 32 * PL, Q = PL / 4;
+    if (fend - fstart + 3 <= PR) {
+        // the common case (a tile of near-uniform weights has ~256 slots): the tile's slots, behind up to 3 slots of
+        // padding, fit one round of PL consecutive slots per lane.  Every particle with offspring marks the FIRST of its
+        // slots with its index (one predicated store, no divergence on the family size); the other slots take the last
+        // mark before them (a running maximum: marks increase with the slot, -1 = no mark), written as 16-byte stores.
         int32_t* const gdst = P.ancestors + (fstart - slot_base);
         const int pad = (int)((reinterpret_cast<uintptr_t>(gdst) >> 2) & 3u);  // window starts 16-byte aligned in global memory
         const int W = fend - fstart + pad;
-        const int rounds = (W + 127) >> 7;
         int4* const w4 = reinterpret_cast<int4*>(out_s);
-        for (int r = 0; r < rounds; ++r) w4[r * 32 + lane] = make_int4(0, 0, 0, 0);
+#pragma unroll
+        for (int j = 0; j < Q; ++j) w4[j * 32 + lane] = make_int4(-1, -1, -1, -1);
         __syncwarp();
         {
             int lo = f_prev;
 #pragma unroll
             for (int k = 0; k < WS_SCAN_ITEMS; ++k) {
                 const int hi = f[k];
-                if (hi > lo) out_s[lo - fstart + pad] = item0 + k + 1;
+                if (hi > lo) out_s[lo - fstart + pad] = item0 + k;
                 lo = hi;
             }
         }
         __syncwarp();
         int32_t* const dst = gdst - pad;
-        int carry = 0;
-        for (int r = 0; r < rounds; ++r) {
-            const int4 v = w4[r * 32 + lane];
-            const int m0 = v.x, m1 = max(m0, v.y), m2 = max(m1, v.z), m3 = max(m2, v.w);
-            int incl = m3;
+        {
+            int mk[PL];
+#pragma unroll
+            for (int j = 0; j < Q; ++j) {
+                const int4 v = w4[lane * Q + j];
+                mk[4 * j] = v.x;
+                mk[4 * j + 1] = v.y;
+                mk[4 * j + 2] = v.z;
+                mk[4 * j + 3] = v.w;
+            }
+#pragma unroll
+            for (int j = 1; j < PL; ++j) mk[j] = max(mk[j], mk[j - 1]);
+            int incl = mk[PL - 1];
 #pragma unroll
             for (int d = 1; d < 32; d <<= 1) {
                 const int t = __shfl_up_sync(0xffffffffu, incl, d);
                 if (lane >= d) incl = max(incl, t);
             }
             int excl = __shfl_up_sync(0xffffffffu, incl, 1);
-            if (lane == 0) excl = 0;
-            excl = max(excl, carry);
-            carry = max(carry, __shfl_sync(0xffffffffu, incl, 31));
-            const int4 o = make_int4(max(m0, excl) - 1, max(m1, excl) - 1, max(m2, excl) - 1, max(m3, excl) - 1);
-            const int p0 = r * 128 + lane * 4;
-            if (p0 >= pad && p0 + 4 <= W) {
-                *reinterpret_cast<int4*>(dst + p0) = o;
+            if (lane == 0) excl = -1;
+#pragma unroll
+            for (int j = 0; j < PL; ++j) mk[j] = max(mk[j], excl);
+            const int p0 = lane * PL;
+            if (p0 >= pad && p0 + PL <= W) {
+#pragma unroll
+                for (int j = 0; j < Q; ++j)
+                    *reinterpret_cast<int4*>(dst + p0 + 4 * j) = make_int4(mk[4 * j], mk[4 * j + 1], mk[4 * j + 2], mk[4 * j + 3]);
             } else {
-                if (p0 >= pad && p0 < W) dst[p0] = o.x;
-                if (p0 + 1 >= pad && p0 + 1 < W) dst[p0 + 1] = o.y;
-                if (p0 + 2 >= pad && p0 + 2 < W) dst[p0 + 2] = o.z;
-                if (p0 + 3 >= pad && p0 + 3 < W) dst[p0 + 3] = o.w;
+#pragma unroll
+                for (int j = 0; j < PL; ++j)
+                    if (p0 + j >= pad && p0 + j < W) dst[p0 + j] = mk[j];
             }
         }
         __syncwarp();
@@ -1777,7 +1827,7 @@ __device__ __forceinline__ void ws_search_warp_tile(const WsScanParams& P, WsSea
 #define WS_SEARCH_ASYNC 1   // next tile's CDF by cp.async into shared memory while this one is searched (1) or loaded when needed (0)
 #endif
 #ifndef WS_SEARCH_MINB
-#define WS_SEARCH_MINB 3
+#define WS_SEARCH_MINB 3   // (4 CTAs per SM fit the 48 KB of shared memory, but at 64 registers the kernel spills and measured slower)
 #endif
 #ifndef WS_SEARCH_GRID
 #define WS_SEARCH_GRID 3   // CTAs per SM launched: persistent warps, each pipelining its tiles (next tile requested while this one is searched)
@@ -1791,13 +1841,14 @@ __device__ __forceinline__ bool ws_gate_closed_identity(const WsScanParams& P) {
     return true;
 }
 #define WS_SEARCH_SMEM_BYTES ((WS_WARPS_PER_CTA * WS_RBUF_SLOTS + WS_CDF_TILE) * 8)
-template <bool EXACT_FP, bool MN>
+template <bool EXACT_FP, bool MN, bool SHR>
 __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_SEARCH_MINB) ws_search_kernel(const __grid_constant__ WsScanParams P) {
     if (ws_gate_closed_identity(P)) return;
 
     // per-warp window: first the slot uniforms of the tile's slot range (Philox mode), then the staged offspring;
     // behind the windows, per warp, the tile-local CDF of the warp's NEXT tile, copied asynchronously while the current
-    // one is searched (the kernel was waiting on these loads: profiles/r2m_ncu_ws_search_kernel_20M.txt)
+    // one is searched (the kernel was waiting on these loads: profiles/r2m_ncu_ws_search_kernel_20M.txt).  The upper half
+    // of a window, above the offspring staging, holds the warp's Philox ring (WsRing) while the ring is in use.
     extern __shared__ __align__(16) unsigned long long search_smem[];
     static_assert(WS_RBUF_SLOTS * 8 >= (WS_EXPAND_CHUNK + 128) * 4 && (WS_RBUF_SLOTS * 8) % 16 == 0, "window too small for the offspring staging");
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1831,9 +1882,16 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_SEARCH_MINB) ws_search_kerne
         if (lane == 31) ow = __ldg(P.tile_words + n_ctiles + ct / WS_TILE_GROUP);   // (32 g + 31 >= ct: the lane is free for the group's prefix)
         pw = (lane == 0 && tile_base % WS_CDF_TILE != 0) ? __ldg(P.cdf_local + tile_base - 1) : 0ull;
     };
-    int tile = blockIdx.x * WS_WARPS_PER_CTA + warp;
-    if (tile < n_tiles) request(tile);
-    for (; tile < n_tiles; tile += warps_total) {
+    // every warp searches a run of consecutive tiles, so that the Philox blocks at the end of one tile's slot range are
+    // still in the warp's ring when the next tile starts
+    static_assert(WS_EXPAND_CHUNK * 4 + WS_RING_BLOCKS * 16 <= WS_RBUF_SLOTS * 8 && 32 * WS_EXPAND_LANE <= WS_EXPAND_CHUNK,
+                  "the ring and the offspring staging share a window");
+    WsRing ring{reinterpret_cast<uint4*>(rbuf + WS_EXPAND_CHUNK / 2), 0u, 0u};
+    const int per_warp = (n_tiles + warps_total - 1) / warps_total;
+    int tile = (blockIdx.x * WS_WARPS_PER_CTA + warp) * per_warp;
+    const int tile_end = min(tile + per_warp, n_tiles);
+    if (tile < tile_end) request(tile);
+    for (; tile < tile_end; ++tile) {
         const int tile_base = tile * WS_SCAN_TILE;
         const int item0 = tile_base + lane * WS_SCAN_ITEMS;
         // global fixed-point CDF of the lane's 8 consecutive particles
@@ -1852,7 +1910,7 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_SEARCH_MINB) ws_search_kerne
         }
         unsigned long long off = ow;
         const unsigned long long pl = pw;
-        if (tile + warps_total < n_tiles) request(tile + warps_total);   // (the lane's slots of cbuf were read above)
+        if (tile + 1 < tile_end) request(tile + 1);   // (the lane's slots of cbuf were read above)
 #pragma unroll
         for (int d = 16; d > 0; d >>= 1) off += __shfl_xor_sync(0xffffffffu, off, d);
         off += cdf_offset;
@@ -1863,8 +1921,8 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_SEARCH_MINB) ws_search_kerne
 #pragma unroll
             for (int k = 0; k < WS_SCAN_ITEMS; ++k) C[k] = (item0 + k < n) ? off + C[k] : 0ull;
         }
-        ws_search_warp_tile<EXACT_FP, MN>(P, X, rbuf, lane, tile_base, C, off + pl, tile != 0,
-                                          WS_INTERIOR_FAST && tile_base + WS_SCAN_TILE < n);
+        ws_search_warp_tile<EXACT_FP, MN, SHR>(P, X, rbuf, lane, tile_base, C, off + pl, tile != 0,
+                                               WS_INTERIOR_FAST && tile_base + WS_SCAN_TILE < n, &ring);
     }
 #else
     for (int tile = blockIdx.x * WS_WARPS_PER_CTA + warp; tile < n_tiles; tile += warps_total) {
@@ -1893,8 +1951,8 @@ __global__ void __launch_bounds__(WS_SCAN_BLOCK, WS_SEARCH_MINB) ws_search_kerne
             // (the particle in front of the first warp tile of a CDF tile lies in the previous CDF tile)
             Cp = (p / WS_CDF_TILE == ct ? offset : offset - __ldg(P.tile_words + ct - 1)) + __ldg(P.cdf_local + p);
         }
-        ws_search_warp_tile<EXACT_FP, MN>(P, X, rbuf, lane, tile_base, C, Cp, tile != 0,
-                                          WS_INTERIOR_FAST && tile_base + WS_SCAN_TILE < n);
+        ws_search_warp_tile<EXACT_FP, MN, SHR>(P, X, rbuf, lane, tile_base, C, Cp, tile != 0,
+                                               WS_INTERIOR_FAST && tile_base + WS_SCAN_TILE < n);
     }
 #endif
 }
@@ -2523,9 +2581,10 @@ cudaError_t ws_launch_search(const WsScanParams& P, cudaStream_t s) {
     int g3 = (int)(ctas < (int64_t)g_sm_count * WS_SEARCH_GRID ? ctas : (int64_t)g_sm_count * WS_SEARCH_GRID);
     if (g3 < 1) g3 = 1;
     const bool exact_fp = P.replay_u != nullptr || P.sorted_u != nullptr;
-    if (exact_fp) ws_search_kernel<true, false><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
-    else if (P.scheme == 2) ws_search_kernel<false, true><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
-    else ws_search_kernel<false, false><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
+    if (exact_fp) ws_search_kernel<true, false, false><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
+    else if (P.scheme == 2) ws_search_kernel<false, true, false><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
+    else if (P.fx_shift >= 32) ws_search_kernel<false, false, true><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);   // N <= 2^29
+    else ws_search_kernel<false, false, false><<<g3, WS_SCAN_BLOCK, WS_SEARCH_SMEM_BYTES, s>>>(P);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     ws_expand_heavy_kernel<<<g_sm_count * 4, 256, 0, s>>>(P);
@@ -2814,11 +2873,13 @@ cudaError_t ws_kernels_init(int device) {
         g_vm_interp_only = v != nullptr && strcmp(v, "interp") == 0;
     }
     // the register file of the fused pass can take most of the SM's shared memory
-    e = cudaFuncSetAttribute(ws_search_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
+    e = cudaFuncSetAttribute(ws_search_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ws_search_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
+    e = cudaFuncSetAttribute(ws_search_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(ws_search_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
+    e = cudaFuncSetAttribute(ws_search_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(ws_search_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_SEARCH_SMEM_BYTES);
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(ws_chain_kernel<true, WS_SCAN_BLOCK>, cudaFuncAttributeMaxDynamicSharedMemorySize, WS_CHAIN_SMEM_BYTES(WS_SCAN_BLOCK));
     if (e != cudaSuccess) return e;

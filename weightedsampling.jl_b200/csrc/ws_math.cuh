@@ -234,9 +234,8 @@ static const double ws_coef_host[WS_CI_COUNT] = {WS_MATH_COEFS(WS_COEF_VALUE)};
 #define WS_K(name) ws_coef_host[WS_CI_##name]
 #endif
 
-// exp(d) for d <= 0 (log-weight minus its maximum): Cody-Waite reduction, degree-11 polynomial.
-// d < -708 (result below the normal range) and d = -inf give 0; NaN gives NaN.
-WS_HD double ws_exp_nonpos(double d) {
+// exp(d) for -708 < d <= 0: Cody-Waite reduction, degree-11 polynomial.  Outside that range the result is garbage.
+WS_HD double ws_exp_nonpos_core(double d) {
     const double MAGIC = 6755399441055744.0;  // 1.5 * 2^52: fma(d, log2e, MAGIC) holds rint(d*log2e) in its low word
     const double t = ws_fma(d, WS_K(EXP_LOG2E), MAGIC);
     const double kd = t - MAGIC;
@@ -255,8 +254,21 @@ WS_HD double ws_exp_nonpos(double d) {
     p = ws_fma(p, r, 1.0);
     p = ws_fma(p, r, 1.0);
     const uint64_t k = (uint64_t)(uint32_t)ws_double_to_bits(t);  // low word of t = k as a two's-complement int32
-    const double v = ws_bits_to_double(ws_double_to_bits(p) + (k << 52));
+    return ws_bits_to_double(ws_double_to_bits(p) + (k << 52));
+}
+
+// exp(d) for d <= 0 (log-weight minus its maximum).
+// d < -708 (result below the normal range) and d = -inf give 0; NaN gives NaN.
+WS_HD double ws_exp_nonpos(double d) {
+    const double v = ws_exp_nonpos_core(d);
     return (d > -708.0) ? v : ((d != d) ? d : 0.0);
+}
+
+// ws_exp_nonpos with NaN sent to 0 as well (one compare instead of two), for callers that convert the result
+// with a saturating NaN -> 0 conversion anyway: d < -708, -inf and NaN give 0.
+WS_HD double ws_exp_nonpos_or0(double d) {
+    const double v = ws_exp_nonpos_core(d);
+    return (d > -708.0) ? v : 0.0;
 }
 
 // a / b for finite a >= 0, b > 0 with rb = RN(1 / b) hoisted by the caller: product, exact residual, one
