@@ -294,11 +294,28 @@ int ws_resample_host(ws_ctx* ctx, const double* weights, int64_t n, int scheme, 
 /* @E(f, state) / expectation(values, weights): sum_i f_i * exp_norm(weights)_i
  * (src/utils.jl:11,45-68).  n_exprs expectations in one pass. */
 int ws_expectation(ws_ctx* ctx, const ws_expr* f, int32_t n_exprs, double* out);
-/* sample(state, n; replace) index draw (src/utils.jl:102-118): n 0-based particle indices
- * drawn with probability exp_norm(weights). */
+/* sample(state, n; replace) index draw (src/utils.jl:102-118): n 0-based GLOBAL particle indices drawn with
+ * probability exp_norm(weights), made on the device.  On one GPU global and local indices are the same.  Collective on
+ * a sharded state: every rank calls it and gets the same n indices.  The draw does not depend on the number of GPUs:
+ * l_i is the current log-weight of global particle i, m = max_i l_i (exact in any reduction order), and the Philox
+ * stream is the context's next stream (one per call, so the ranks stay in lockstep).
+ *   With replacement:  q_i = rint(exp(l_i - m) 2^52) (0 for NaN or -inf l_i),  Q_j = sum_{i<=j} q_i and T = Q_{N-1}
+ *     in exact integers (128-bit);  r_k = the 128-bit integer of Philox block (k, stream, seed),
+ *     t_k = floor(r_k T / 2^128),  index_k = min{ j : Q_j > t_k }.  Every draw lands on a particle with q_j > 0.
+ *     A particle whose weight is below 2^-53 of the largest is never drawn.
+ *   Without replacement (n <= N):  key_i = l_i - log(E_i), E_i the standard exponential of Philox block
+ *     (i, stream, seed) (ws_randexp).  The n largest keys in descending order, equal keys to the lower index;
+ *     particles with a NaN or -inf log-weight rank below every finite key, ordered by index.
+ * WS_ENUMERIC if the largest log-weight is not finite (all -inf or NaN, or +inf); WS_EINVAL for n <= 0 and for
+ * n > N without replacement.  Only the n draws cross PCIe.  (csrc/ws_math.cuh: ws_sample_q, ws_sample_target,
+ * ws_sample_key; csrc/ws_kernels_stats.cu) */
 int ws_sample_indices(ws_ctx* ctx, int64_t n_draws, int replace, int64_t* indices_out);
 /* rows `indices` of column id -> host (plane-major, n_idx per plane). */
 int ws_col_download_rows(ws_ctx* ctx, int32_t id, const int64_t* indices, int64_t n_idx, double* host_out);
+/* rows of GLOBAL particle indices (0 <= index < N) of column id -> host (plane-major, n_idx per plane).  Collective on
+ * a sharded state: each rank reads the rows it owns and every rank gets all n_idx rows, bit for bit.  On one GPU the
+ * same as ws_col_download_rows. */
+int ws_col_download_global_rows(ws_ctx* ctx, int32_t id, const int64_t* global_indices, int64_t n_idx, double* host_out);
 
 /* ---- MH moves (src/transformers.jl:588-623, src/move_kernels.jl:189-253) ------------------ */
 #define WS_PROPOSAL_RW 0

@@ -555,13 +555,16 @@ function describe_plane(state::DeviceState, name::Symbol, comp::Integer=0)
                             ctx(state), 1, Ref(Int32(id)), Ref(Int32(comp)), out, ess))
     out[], ess[]
 end
-"`sample(state, n; replace)` (utils.jl:102-118): 1-based particle indices and the rows of one column"
+"""`sample(state, n; replace)` (utils.jl:102-118): 1-based GLOBAL particle indices and the rows of one column, drawn on
+the device.  Collective on a sharded state: every rank calls it and gets the same indices and rows.
+(Not executed in this repository's test suite: there is no Julia toolchain here.)"""
 function sample_rows(state::DeviceState, name::Symbol, n::Integer; replace::Bool=true)
     idx = Vector{Int64}(undef, n)
     check(ctx(state), ccall((:ws_sample_indices, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Ptr{Int64}), ctx(state), n, replace, idx))
     id, w = lookup(state.store, name)
     rows = Matrix{Float64}(undef, n, w)
-    check(ctx(state), ccall((:ws_col_download_rows, LIB), Cint, (Ptr{Cvoid}, Int32, Ptr{Int64}, Int64, Ptr{Float64}), ctx(state), id, idx, n, rows))
+    check(ctx(state), ccall((:ws_col_download_global_rows, LIB), Cint, (Ptr{Cvoid}, Int32, Ptr{Int64}, Int64, Ptr{Float64}),
+                            ctx(state), id, idx, n, rows))
     idx .+ 1, rows
 end
 function marginal_diversity(state::DeviceState, targets::Vector{Symbol})               # transformers.jl:560-565

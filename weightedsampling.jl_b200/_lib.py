@@ -153,6 +153,7 @@ SIGNATURES = {
     "ws_expectation": (C.c_int, [_ctx, _ep, C.c_int32, _dp]),
     "ws_sample_indices": (C.c_int, [_ctx, C.c_int64, C.c_int, C.c_void_p]),
     "ws_col_download_rows": (C.c_int, [_ctx, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
+    "ws_col_download_global_rows": (C.c_int, [_ctx, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "ws_move": (C.c_int, [_ctx, C.POINTER(ws_move_spec), C.POINTER(ws_move_info)]),
     "ws_marginal_diversity": (C.c_int, [_ctx, C.c_int32, _i32p, _i32p, _dp]),
     "ws_score_logpdf": (C.c_int, [_ctx, C.c_int64, C.c_void_p]),

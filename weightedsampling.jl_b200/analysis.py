@@ -1,6 +1,6 @@
 """Post-run analysis surface (src/utils.jl): ``exp_norm``, ``expectation``, ``@E``, ``log_evidence``,
 ``sample``.  Reductions over the particles run on the device (``ws_exp_norm``, ``ws_expectation``,
-``ws_log_evidence``); only their small results come back to the host.
+``ws_log_evidence``, ``ws_sample_indices``); only their small results come back to the host.
 """
 from __future__ import annotations
 
@@ -120,21 +120,26 @@ def expectation(values, state):
 
 
 def sample(state, n, replace=True):
-    """``sample(state, n; replace=true)`` (utils.jl:102-118) -> pandas DataFrame of n particles."""
+    """``sample(state, n; replace=true)`` (utils.jl:102-118) -> pandas DataFrame of n particles.
+
+    The indices are drawn on the device (``ws_sample_indices``) and only the n drawn rows come to the host.  On a
+    sharded state the call is collective: every rank must call it, and every rank gets the same DataFrame."""
     import pandas as pd
     st = state.store
     n = int(n)
+    n_all = getattr(st, "n_global", st.n)
     if n <= 0:
         raise ValueError("Number of samples must be positive")
-    if not replace and n > st.n:
-        raise ValueError(f"Cannot sample {n} particles without replacement from {st.n} particles")
+    if not replace and n > n_all:
+        raise ValueError(f"Cannot sample {n} particles without replacement from {n_all} particles")
     idx = np.empty(n, dtype=np.int64)
     st._call("ws_sample_indices", n, int(bool(replace)), idx.ctypes.data_as(C.c_void_p))
+    rows_call = "ws_col_download_global_rows" if getattr(st, "nranks", 1) > 1 else "ws_col_download_rows"
     data = {}
     for name in st.colnames():
         cid, width = st._lookup(name)
         rows = np.empty((width, n), dtype=np.float64)
-        st._call("ws_col_download_rows", cid, idx.ctypes.data_as(C.c_void_p), n, rows.ctypes.data_as(C.c_void_p))
+        st._call(rows_call, cid, idx.ctypes.data_as(C.c_void_p), n, rows.ctypes.data_as(C.c_void_p))
         data[name] = rows[0] if width == 1 else list(np.ascontiguousarray(rows.T))
     return pd.DataFrame(data)
 

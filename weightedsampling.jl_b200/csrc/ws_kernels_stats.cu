@@ -11,6 +11,10 @@
 //   8 x (histogram of the next key byte | pick the byte where the running mass first exceeds h)
 //   pass F   neighbours of the selected value: largest smaller value, smallest weight at the value
 // All of it is HBM streaming work: 8 (x) + 8 (q) bytes per particle and pass.
+//
+// The second half of the file is sample(state, n; replace) (src/utils.jl:102-118), the draw include/wsb200.h defines
+// above ws_sample_indices.  It reuses the pick step of the radix select and the same cross-rank hooks.
+#include <algorithm>
 #include <vector>
 #include <string.h>
 #include "ws_internal.h"
@@ -176,19 +180,26 @@ __global__ void __launch_bounds__(256) ws_stats_hist_kernel(const double* __rest
     }
 }
 
-__global__ void ws_stats_pick_kernel(int pass, unsigned long long* __restrict__ state, unsigned long long* __restrict__ hist) {
-    if (threadIdx.x != 0) return;
-    unsigned long long below = state[1];
-    const unsigned long long hh = state[2];
+// the bin b where the running mass `below` + hist[0..b] first exceeds hh (-1: never); `below` is advanced to the mass
+// of the bins before it and *mass gets the bin's own mass
+__device__ __forceinline__ int ws_radix_pick(unsigned long long& below, unsigned long long hh, const unsigned long long* hist,
+                                             unsigned long long* mass) {
     int pick = -1;
     for (int b = 0; b < 256; ++b) {
         const unsigned long long c = hist[b];
         if (pick < 0 && c != 0ull && below + c > hh) {
             pick = b;
-            state[3] = c;
+            *mass = c;
         }
         if (pick < 0) below += c;
     }
+    return pick;
+}
+
+__global__ void ws_stats_pick_kernel(int pass, unsigned long long* __restrict__ state, unsigned long long* __restrict__ hist) {
+    if (threadIdx.x != 0) return;
+    unsigned long long below = state[1];
+    int pick = ws_radix_pick(below, state[2], hist, &state[3]);
     if (pick < 0) {
         state[4] = 1ull;  // the running mass never exceeds h: quantile() returns the maximum
         pick = 255;
@@ -390,4 +401,334 @@ cudaError_t ws_stats_plane(const double* x, const unsigned long long* q, int64_t
     return cudaSuccess;
 }
 
+// =========================================================================================================
+// sample(state, n; replace) on the device
+//
+// With replacement (exact inversion of the integer CDF of q_i = ws_sample_q(l_i, m)):
+//   ws_sample_cdf_tiles_kernel   q -> tile-local inclusive prefix P (8 B per particle) and one sum per tile of 2048
+//   ws_sample_offsets_kernel     one CTA: exclusive 128-bit scan of the tile sums, the shard's mass T_r at the end
+//   ws_sample_draw_kernel        one thread per draw: Philox -> t_k; skip unless t_k falls in [O_r, O_r + T_r);
+//                                binary search over the tile offsets, then inside the tile -> global index + 1
+//   sharded: the T_r travel with one allgather, the draws with one integer all-reduce (each draw has one owner)
+// Without replacement (the n largest Gumbel keys, ties to the lower global index):
+//   ws_sample_keys_kernel        64-bit key image per particle
+//   8 x (ws_sample_hist_kernel | ws_sample_pick_kernel)   radix select over COUNT histograms: the n-th largest key
+//   4 x (the same over the index bytes of the particles at that key)  the lowest-index ones taken at a tie
+//   ws_sample_compact_kernel     the n winners (key, global index); the host sorts them (n log n, n << N)
+// Every count and mass is an integer, so the result does not depend on the grid or on the number of ranks.
+// =========================================================================================================
+#define WS_SMP_TILE 2048      // particles per CDF tile: a tile sum <= 2048 (2^52 + 1) stays below 2^63
+#define WS_SMP_PER_THREAD 8   // consecutive particles per thread (256 threads)
+typedef unsigned __int128 ws_smp_u128;
 
+__global__ void __launch_bounds__(256) ws_sample_cdf_tiles_kernel(const double* __restrict__ logw, int64_t n, double m,
+                                                                   unsigned long long* __restrict__ P,
+                                                                   unsigned long long* __restrict__ tile_sum) {
+    __shared__ unsigned long long warp_tot[8];
+    const int64_t base = (int64_t)blockIdx.x * WS_SMP_TILE + (int64_t)threadIdx.x * WS_SMP_PER_THREAD;
+    unsigned long long pre[WS_SMP_PER_THREAD];
+    unsigned long long s = 0ull;
+#pragma unroll
+    for (int j = 0; j < WS_SMP_PER_THREAD; ++j) {
+        const int64_t i = base + j;
+        s += i < n ? ws_sample_q(logw[i], m) : 0ull;
+        pre[j] = s;
+    }
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    unsigned long long x = s;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const unsigned long long y = __shfl_up_sync(0xffffffffu, x, d);
+        if (lane >= d) x += y;
+    }
+    if (lane == 31) warp_tot[warp] = x;
+    __syncthreads();
+    unsigned long long before = x - s;
+    for (int w = 0; w < warp; ++w) before += warp_tot[w];
+#pragma unroll
+    for (int j = 0; j < WS_SMP_PER_THREAD; ++j)
+        if (base + j < n) P[base + j] = before + pre[j];
+    if (threadIdx.x == 255) tile_sum[blockIdx.x] = before + s;
+}
+
+// off[b] = sum of the tile sums before b (128-bit), off[n_tiles] = the shard's total T_r
+__global__ void __launch_bounds__(1024) ws_sample_offsets_kernel(const unsigned long long* __restrict__ tile_sum, int64_t n_tiles,
+                                                                  ws_smp_u128* __restrict__ off) {
+    __shared__ ws_smp_u128 sm[1024];
+    const int t = threadIdx.x;
+    const int64_t per = (n_tiles + 1023) / 1024;
+    const int64_t b0 = (int64_t)t * per, b1 = b0 + per < n_tiles ? b0 + per : n_tiles;
+    ws_smp_u128 s = 0;
+    for (int64_t b = b0; b < b1; ++b) s += tile_sum[b];
+    sm[t] = s;
+    __syncthreads();
+    for (int d = 1; d < 1024; d <<= 1) {
+        const ws_smp_u128 v = t >= d ? sm[t - d] : (ws_smp_u128)0;
+        __syncthreads();
+        sm[t] += v;
+        __syncthreads();
+    }
+    ws_smp_u128 run = sm[t] - s;
+    for (int64_t b = b0; b < b1; ++b) {
+        off[b] = run;
+        run += tile_sum[b];
+    }
+    if (t == 1023) off[n_tiles] = sm[1023];
+}
+
+__global__ void __launch_bounds__(256) ws_sample_draw_kernel(const unsigned long long* __restrict__ P, const ws_smp_u128* __restrict__ off,
+                                                              int64_t n_tiles, int64_t n, int64_t offset, ws_u128 T, ws_u128 O,
+                                                              int64_t n_draws, uint64_t stream, uint64_t seed,
+                                                              unsigned long long* __restrict__ out) {
+    const int64_t k = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (k >= n_draws) return;
+    const ws_u128 t = ws_sample_target((uint64_t)k, stream, seed, T);
+    const ws_smp_u128 tt = ((ws_smp_u128)t.hi << 64) | t.lo, o = ((ws_smp_u128)O.hi << 64) | O.lo;
+    if (tt < o || tt - o >= off[n_tiles]) {  // another rank's particle
+        out[k] = 0ull;
+        return;
+    }
+    const ws_smp_u128 loc = tt - o;
+    int64_t lo = 0, hi = n_tiles - 1;  // the last tile whose offset is <= loc (it has a non-zero sum)
+    while (lo < hi) {
+        const int64_t mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= loc) lo = mid; else hi = mid - 1;
+    }
+    const unsigned long long w = (unsigned long long)(loc - off[lo]);
+    int64_t a = lo * WS_SMP_TILE, e = (a + WS_SMP_TILE < n ? a + WS_SMP_TILE : n) - 1;  // the first j with P[j] > w
+    while (a < e) {
+        const int64_t mid = (a + e) >> 1;
+        if (P[mid] > w) e = mid; else a = mid + 1;
+    }
+    out[k] = (unsigned long long)(offset + a + 1);
+}
+
+__global__ void __launch_bounds__(256) ws_sample_keys_kernel(const double* __restrict__ logw, int64_t n, int64_t offset, uint64_t stream,
+                                                              uint64_t seed, unsigned long long* __restrict__ keys) {
+    const int64_t stride = (int64_t)gridDim.x * 256;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += stride)
+        keys[i] = ws_sample_key(logw[i], (uint64_t)(offset + i), stream, seed);
+}
+
+// state: [0] key prefix (left-aligned; after pass 7 the selected key), [1] count below the prefix range, [2] the rank h
+// to select (ascending), [3] count in the selected bin, [5] index prefix (passes 8..11), [6] 1: every particle at the
+// selected key is taken (the index passes are skipped), [7] 1: a histogram never crossed h (cannot happen)
+#define WS_SMP_KEY_PASSES 8
+#define WS_SMP_PASSES 12   // + 4 bytes of the global index (N < 2^31)
+__global__ void __launch_bounds__(256) ws_sample_hist_kernel(const unsigned long long* __restrict__ keys, int64_t n, int64_t offset, int pass,
+                                                              const unsigned long long* __restrict__ state,
+                                                              unsigned long long* __restrict__ hist /* [256] */) {
+    __shared__ unsigned int h[8][256];
+    if (pass >= WS_SMP_KEY_PASSES && state[6] != 0ull) return;
+    for (int k = threadIdx.x; k < 8 * 256; k += 256) (&h[0][0])[k] = 0u;
+    __syncthreads();
+    const int warp = threadIdx.x >> 5;
+    const int64_t stride = (int64_t)gridDim.x * 256;
+    if (pass < WS_SMP_KEY_PASSES) {
+        const unsigned long long prefix = state[0];
+        const int shift = 56 - 8 * pass;
+        const unsigned long long himask = pass == 0 ? 0ull : (~0ull << (shift + 8));
+        for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) {
+            const unsigned long long key = keys[i];
+            if ((key & himask) == prefix) atomicAdd(&h[warp][(key >> shift) & 0xFFull], 1u);
+        }
+    } else {
+        const unsigned long long sel = state[0], prefix = state[5];
+        const int shift = 24 - 8 * (pass - WS_SMP_KEY_PASSES);
+        const unsigned long long himask = ~0ull << (shift + 8);
+        for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) {
+            if (keys[i] != sel) continue;
+            const unsigned long long g = (unsigned long long)(offset + i);
+            if ((g & himask) == prefix) atomicAdd(&h[warp][(g >> shift) & 0xFFull], 1u);
+        }
+    }
+    __syncthreads();
+    unsigned long long s = 0ull;
+    for (int w = 0; w < 8; ++w) s += h[w][threadIdx.x];
+    if (s != 0ull) atomicAdd(hist + threadIdx.x, s);
+}
+
+__global__ void ws_sample_pick_kernel(int pass, unsigned long long* __restrict__ state, unsigned long long* __restrict__ hist) {
+    if (threadIdx.x != 0) return;
+    if (pass >= WS_SMP_KEY_PASSES && state[6] != 0ull) return;  // nothing was counted
+    unsigned long long below = state[1], mass = 0ull;
+    int pick = ws_radix_pick(below, state[2], hist, &mass);
+    if (pick < 0) {  // the counts sum to the number of candidates, which always exceeds h
+        state[7] = 1ull;
+        pick = 0;
+    }
+    if (pass < WS_SMP_KEY_PASSES) {
+        state[0] |= (unsigned long long)pick << (56 - 8 * pass);
+        state[1] = below;
+        state[3] = mass;
+        if (pass == WS_SMP_KEY_PASSES - 1) {
+            // the particles at the selected key hold ascending ranks [below, below + mass); ranks >= h are taken
+            const unsigned long long h = state[2];
+            if (below == h) {
+                state[6] = 1ull;
+            } else {  // take the (below + mass - h) lowest global indices among them: select the last one
+                state[2] = below + mass - h - 1ull;
+                state[1] = 0ull;
+            }
+        }
+    } else {
+        state[5] |= (unsigned long long)pick << (24 - 8 * (pass - WS_SMP_KEY_PASSES));
+        state[1] = below;
+    }
+    for (int b = 0; b < 256; ++b) hist[b] = 0ull;
+}
+
+__global__ void __launch_bounds__(256) ws_sample_compact_kernel(const unsigned long long* __restrict__ keys, int64_t n, int64_t offset,
+                                                                 const unsigned long long* __restrict__ state,
+                                                                 unsigned long long* __restrict__ count,
+                                                                 unsigned long long* __restrict__ pairs, int64_t cap) {
+    const unsigned long long sel = state[0], gmax = state[6] != 0ull ? ~0ull : state[5];
+    const int64_t stride = (int64_t)gridDim.x * 256;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < n; i += stride) {
+        const unsigned long long key = keys[i], g = (unsigned long long)(offset + i);
+        if (key > sel || (key == sel && g <= gmax)) {
+            const unsigned long long pos = atomicAdd(count, 1ull);
+            if (pos < (unsigned long long)cap) {
+                pairs[2 * pos] = key;
+                pairs[2 * pos + 1] = g;
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) ws_sample_scatter_kernel(const double* __restrict__ src, const int64_t* __restrict__ pos, int64_t n,
+                                                                 double* __restrict__ dst) {
+    const int64_t j = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (j < n) dst[pos[j]] = src[j];
+}
+
+static size_t smp_up(size_t b) { return (b + 255) & ~(size_t)255; }
+static int64_t smp_tiles(int64_t n) { return (n + WS_SMP_TILE - 1) / WS_SMP_TILE; }
+
+size_t ws_sample_scratch_bytes(int64_t n, int64_t n_draws, int replace) {
+    const int64_t t = smp_tiles(n);
+    if (replace)
+        return smp_up(8 * (size_t)n) + smp_up(8 * (size_t)t) + smp_up(16 * (size_t)(t + 1)) + smp_up(8 * (size_t)n_draws);
+    return smp_up(8 * (size_t)n) + smp_up(8 * 256) + smp_up(8 * 8) + smp_up(8) + smp_up(16 * (size_t)n_draws);
+}
+
+static cudaError_t sample_with_replacement(const double* logw, int64_t n, int64_t offset, double m, uint64_t seed, uint64_t stream,
+                                           int64_t n_draws, char* dp, cudaStream_t s, int64_t* out, int* n_launches,
+                                           int64_t* d2h_bytes, const WsStatsComm* comm) {
+    const int64_t tiles = smp_tiles(n);
+    unsigned long long* P = (unsigned long long*)dp;
+    unsigned long long* tsum = (unsigned long long*)(dp + smp_up(8 * (size_t)n));
+    ws_smp_u128* off = (ws_smp_u128*)((char*)tsum + smp_up(8 * (size_t)tiles));
+    unsigned long long* d_out = (unsigned long long*)((char*)off + smp_up(16 * (size_t)(tiles + 1)));
+    cudaError_t e;
+    ws_sample_cdf_tiles_kernel<<<(unsigned)tiles, 256, 0, s>>>(logw, n, m, P, tsum);
+    ws_sample_offsets_kernel<<<1, 1024, 0, s>>>(tsum, tiles, off);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    ws_smp_u128 Tr = 0;
+    if ((e = cudaMemcpyAsync(&Tr, off + tiles, 16, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+    *d2h_bytes += 16;
+    ws_smp_u128 O = 0, T = Tr;
+    if (comm != nullptr) {  // the ranks' masses in rank order: this rank's draws are the t in [O, O + T_r)
+        const unsigned long long mine[2] = {(unsigned long long)(Tr >> 64), (unsigned long long)Tr};
+        std::vector<unsigned long long> all(2 * (size_t)comm->nranks);
+        if (comm->allgather_words(comm->ctx, mine, 2, all.data()) != 0) return cudaErrorUnknown;
+        *d2h_bytes += 16 * comm->nranks;
+        T = 0;
+        for (int r = 0; r < comm->nranks; ++r) {
+            const ws_smp_u128 v = ((ws_smp_u128)all[2 * r] << 64) | all[2 * r + 1];
+            if (r < comm->rank) O += v;
+            T += v;
+        }
+    }
+    ws_u128 T2, O2;
+    T2.hi = (uint64_t)(T >> 64);
+    T2.lo = (uint64_t)T;
+    O2.hi = (uint64_t)(O >> 64);
+    O2.lo = (uint64_t)O;
+    ws_sample_draw_kernel<<<(unsigned)((n_draws + 255) / 256), 256, 0, s>>>(P, off, tiles, n, offset, T2, O2, n_draws, stream, seed, d_out);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    *n_launches += 3;
+    if (comm != nullptr && comm->allreduce_u64_device(comm->ctx, d_out, (size_t)n_draws) != 0) return cudaErrorUnknown;
+    if ((e = cudaMemcpyAsync(out, d_out, 8 * (size_t)n_draws, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+    *d2h_bytes += 8 * n_draws;
+    for (int64_t k = 0; k < n_draws; ++k) {
+        if (out[k] <= 0) return cudaErrorInvalidValue;  // no rank owned the draw
+        out[k] -= 1;
+    }
+    return cudaSuccess;
+}
+
+static cudaError_t sample_without_replacement(const double* logw, int64_t n, int64_t offset, int64_t n_global, uint64_t seed,
+                                              uint64_t stream, int64_t n_draws, char* dp, cudaStream_t s, int64_t* out,
+                                              int* n_launches, int64_t* d2h_bytes, const WsStatsComm* comm) {
+    unsigned long long* keys = (unsigned long long*)dp;
+    unsigned long long* d_hist = (unsigned long long*)(dp + smp_up(8 * (size_t)n));
+    unsigned long long* d_state = (unsigned long long*)((char*)d_hist + smp_up(8 * 256));
+    unsigned long long* d_count = (unsigned long long*)((char*)d_state + smp_up(8 * 8));
+    unsigned long long* d_pairs = (unsigned long long*)((char*)d_count + smp_up(8));
+    const int g = stats_grid(n);
+    cudaError_t e;
+    ws_sample_keys_kernel<<<g, 256, 0, s>>>(logw, n, offset, stream, seed, keys);
+    const unsigned long long st0[8] = {0ull, 0ull, (unsigned long long)(n_global - n_draws), 0ull, 0ull, 0ull, 0ull, 0ull};
+    if ((e = cudaMemcpyAsync(d_state, st0, sizeof(st0), cudaMemcpyHostToDevice, s)) != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(d_hist, 0, 8 * 256, s)) != cudaSuccess) return e;
+    if ((e = cudaMemsetAsync(d_count, 0, 8, s)) != cudaSuccess) return e;
+    for (int pass = 0; pass < WS_SMP_PASSES; ++pass) {
+        ws_sample_hist_kernel<<<g, 256, 0, s>>>(keys, n, offset, pass, d_state, d_hist);
+        if (comm != nullptr && comm->allreduce_u64_device(comm->ctx, d_hist, 256) != 0) return cudaErrorUnknown;  // exact counts
+        ws_sample_pick_kernel<<<1, 32, 0, s>>>(pass, d_state, d_hist);
+    }
+    ws_sample_compact_kernel<<<g, 256, 0, s>>>(keys, n, offset, d_state, d_count, d_pairs, n_draws);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    *n_launches += 2 + 2 * WS_SMP_PASSES;
+    unsigned long long h_state[8], cnt = 0ull;
+    if ((e = cudaMemcpyAsync(h_state, d_state, sizeof(h_state), cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+    if ((e = cudaMemcpyAsync(&cnt, d_count, 8, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+    if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+    *d2h_bytes += sizeof(h_state) + 8;
+    if (h_state[7] != 0ull || cnt > (unsigned long long)n_draws) return cudaErrorInvalidValue;
+    std::vector<unsigned long long> pairs(2 * (size_t)cnt);
+    if (cnt > 0ull) {
+        if ((e = cudaMemcpyAsync(pairs.data(), d_pairs, 16 * (size_t)cnt, cudaMemcpyDeviceToHost, s)) != cudaSuccess) return e;
+        if ((e = cudaStreamSynchronize(s)) != cudaSuccess) return e;
+        *d2h_bytes += 16 * (int64_t)cnt;
+    }
+    if (comm != nullptr) {  // every rank's winners, in rank order
+        std::vector<unsigned long long> counts((size_t)comm->nranks);
+        if (comm->allgather_words(comm->ctx, &cnt, 1, counts.data()) != 0) return cudaErrorUnknown;
+        const unsigned long long mx = *std::max_element(counts.begin(), counts.end());
+        std::vector<unsigned long long> mine(2 * (size_t)mx, 0ull), all(2 * (size_t)mx * comm->nranks);
+        std::copy(pairs.begin(), pairs.end(), mine.begin());
+        if (mx > 0ull && comm->allgather_words(comm->ctx, mine.data(), 2 * (size_t)mx, all.data()) != 0) return cudaErrorUnknown;
+        *d2h_bytes += 8 * comm->nranks * (1 + 2 * (int64_t)mx);
+        pairs.clear();
+        for (int r = 0; r < comm->nranks; ++r)
+            pairs.insert(pairs.end(), all.begin() + 2 * (size_t)mx * r, all.begin() + 2 * (size_t)mx * r + 2 * (size_t)counts[r]);
+    }
+    if ((int64_t)(pairs.size() / 2) != n_draws) return cudaErrorInvalidValue;
+    std::vector<std::pair<unsigned long long, unsigned long long>> kv((size_t)n_draws);
+    for (int64_t k = 0; k < n_draws; ++k) kv[(size_t)k] = {pairs[2 * (size_t)k], pairs[2 * (size_t)k + 1]};
+    std::sort(kv.begin(), kv.end(), [](const std::pair<unsigned long long, unsigned long long>& a,
+                                       const std::pair<unsigned long long, unsigned long long>& b) {
+        return a.first != b.first ? a.first > b.first : a.second < b.second;  // descending key, then lower index
+    });
+    for (int64_t k = 0; k < n_draws; ++k) out[k] = (int64_t)kv[(size_t)k].second;
+    return cudaSuccess;
+}
+
+cudaError_t ws_sample_draw(const double* logw, int64_t n, int64_t offset, int64_t n_global, double m, uint64_t seed, uint64_t stream,
+                           int64_t n_draws, int replace, void* d_scratch, cudaStream_t s, int64_t* out, int* n_launches,
+                           int64_t* d2h_bytes, const WsStatsComm* comm) {
+    *n_launches = 0;
+    if (replace)
+        return sample_with_replacement(logw, n, offset, m, seed, stream, n_draws, (char*)d_scratch, s, out, n_launches, d2h_bytes, comm);
+    return sample_without_replacement(logw, n, offset, n_global, seed, stream, n_draws, (char*)d_scratch, s, out, n_launches, d2h_bytes,
+                                      comm);
+}
+
+cudaError_t ws_sample_scatter_rows(const double* src, const int64_t* pos, int64_t n, double* dst, cudaStream_t s) {
+    ws_sample_scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(src, pos, n, dst);
+    return cudaGetLastError();
+}

@@ -476,6 +476,72 @@ WS_HD unsigned long long ws_spacing_of_slot(uint64_t k, int mn_shift, uint64_t s
 }
 
 // ---------------------------------------------------------------------------
+// sample(state, n; replace) (src/utils.jl:102-118), drawn on the device (csrc/ws_kernels_stats.cu).  Every piece is a
+// function of the particle's GLOBAL index, its log-weight and the global maximum m only, so the draw does not depend
+// on the number of ranks; the CPU harness evaluates the same code to regenerate the device values bit for bit.
+// ---------------------------------------------------------------------------
+#define WS_SAMPLE_Q_SCALE 4503599627370496.0 /* 2^52, relative to the largest weight */
+struct ws_u128 {
+    uint64_t hi, lo;
+};
+// with replacement: integer weight q_i = rint(exp(l_i - m) 2^52); NaN, -inf and l_i - m < -708 give 0
+WS_HD uint64_t ws_sample_q(double l, double m) {
+    const double v = ws_exp_nonpos_or0(l - m) * WS_SAMPLE_Q_SCALE;
+#if defined(__CUDA_ARCH__)
+    return __double2ull_rn(v);
+#else
+    return (uint64_t)llrint(v);
+#endif
+}
+WS_HD void ws_mul64(uint64_t a, uint64_t b, uint64_t& hi, uint64_t& lo) {
+#if defined(__CUDA_ARCH__)
+    lo = a * b;
+    hi = __umul64hi(a, b);
+#else
+    const unsigned __int128 p = (unsigned __int128)a * b;
+    lo = (uint64_t)p;
+    hi = (uint64_t)(p >> 64);
+#endif
+}
+// draw k's target t_k = floor(r_k T / 2^128), r_k = the 128-bit integer (x, y, z, w) of Philox block (k, stream, seed);
+// t_k < T, and the draw is index_k = min{ j : Q_j > t_k } over the exact integer CDF Q of the q_i
+WS_HD ws_u128 ws_sample_target(uint64_t k, uint64_t stream, uint64_t seed, ws_u128 T) {
+    const ws_u32x4 r = ws_philox4x32_10(k, stream, seed);
+    const uint64_t a1 = ((uint64_t)r.x << 32) | r.y, a0 = ((uint64_t)r.z << 32) | r.w;
+    uint64_t h11, l11, h10, l10, h01, l01, h00, l00;
+    ws_mul64(a1, T.hi, h11, l11);
+    ws_mul64(a1, T.lo, h10, l10);
+    ws_mul64(a0, T.hi, h01, l01);
+    ws_mul64(a0, T.lo, h00, l00);
+    (void)l00;
+    // bits 64..127 of the product: h00 + l10 + l01, whose carries (0..2) go to bits 128..
+    uint64_t mid = h00 + l10;
+    uint64_t carry = mid < l10 ? 1ull : 0ull;
+    mid += l01;
+    carry += mid < l01 ? 1ull : 0ull;
+    ws_u128 t;
+    t.lo = l11 + h10;
+    uint64_t c2 = t.lo < h10 ? 1ull : 0ull;
+    t.lo += h01;
+    c2 += t.lo < h01 ? 1ull : 0ull;
+    t.lo += carry;
+    c2 += t.lo < carry ? 1ull : 0ull;
+    t.hi = h11 + c2;
+    return t;
+}
+// without replacement: the Gumbel / Efraimidis-Spirakis key  key_i = l_i - log(E_i),  E_i = ws_randexp(i, stream, seed);
+// the n largest keys are an exact weighted draw without replacement, in descending order distributed like successive
+// draws.  E_i = 0 (u = 1, probability 2^-53) is read as 2^-54, half the smallest positive value, to stay in the domain
+// of ws_log_pos.  Returned as its order-preserving 64-bit image; a NaN or infinite l_i gives 0, below every finite key.
+WS_HD uint64_t ws_sample_key(double l, uint64_t i, uint64_t stream, uint64_t seed) {
+    if (!(fabs(l) <= 1.7976931348623157e308)) return 0ull;
+    double e = ws_randexp(i, stream, seed);
+    if (!(e > 0.0)) e = 5.551115123125783e-17;  // 2^-54
+    const uint64_t b = ws_double_to_bits(l - ws_log_pos(e));
+    return (b >> 63) ? ~b : (b | 0x8000000000000000ull);
+}
+
+// ---------------------------------------------------------------------------
 // log densities
 // ---------------------------------------------------------------------------
 WS_HD double ws_normal_logpdf(double x, double mu, double sigma) {

@@ -3179,6 +3179,36 @@ extern "C" int ws_expectation(ws_ctx* c, const ws_expr* f, int32_t n_exprs, doub
     return WS_OK;
 }
 
+// rows `d_idx` (n_idx local row indices on the device) of plane k of column `col` -> d_out: the requested rows are traced
+// back through the genealogy when the plane is behind (n_idx chains, not n); `rows` is scratch for the traced indices
+static int gather_rows_traced(ws_ctx* c, const Column& col, int k, const int64_t* d_idx, int64_t n_idx, TempBuf& rows, double* d_out) {
+    const int64_t* use = d_idx;
+    if (col.stale[k]) {
+        if (rows.p == nullptr) CK(c, cudaMalloc(&rows.p, sizeof(int64_t) * (size_t)n_idx));
+        const int64_t* start = d_idx;
+        int64_t from = c->epoch;
+        while (from > col.ep[k]) {
+            WsComposeParams P;
+            memset(&P, 0, sizeof(P));
+            P.n = n_idx;
+            P.n_rows = c->n;
+            while (from > col.ep[k] && P.n_chain < WS_COMPOSE_MAX_CHAIN) {
+                const int32_t* a = anc_of_event(c, from);
+                if (a == nullptr) return fail(c, WS_EINVAL, "genealogy: ancestors of event %lld were released", (long long)from);
+                P.chain[P.n_chain++] = a;
+                --from;
+            }
+            CK(c, ws_launch_compose_rows(P, (int64_t*)rows.p, start, c->stream));
+            c->stats.kernel_launches++;
+            start = (const int64_t*)rows.p;
+        }
+        use = (const int64_t*)rows.p;
+    }
+    CK(c, ws_launch_gather_rows(col.front[k], use, n_idx, d_out, c->stream));
+    c->stats.kernel_launches++;
+    return WS_OK;
+}
+
 extern "C" int ws_col_download_rows(ws_ctx* c, int32_t id, const int64_t* indices, int64_t n_idx, double* host_out) {
     if (!c || !indices || !host_out || n_idx <= 0) return c ? fail(c, WS_EINVAL, "ws_col_download_rows: bad arguments") : WS_EINVAL;
     if (id < 0 || id >= (int32_t)c->cols.size()) return fail(c, WS_EINVAL, "unknown column id %d", id);
@@ -3192,81 +3222,90 @@ extern "C" int ws_col_download_rows(ws_ctx* c, int32_t id, const int64_t* indice
     CK(c, cudaMemcpyAsync(idx.p, indices, sizeof(int64_t) * (size_t)n_idx, cudaMemcpyHostToDevice, c->stream));
     const Column& col = c->cols[id];
     for (int k = 0; k < col.width; ++k) {
-        const int64_t* use = (const int64_t*)idx.p;
-        if (col.stale[k]) {
-            // trace the requested rows back through the genealogy (n_idx chains, not n)
-            if (rows.p == nullptr) CK(c, cudaMalloc(&rows.p, sizeof(int64_t) * (size_t)n_idx));
-            const int64_t* start = (const int64_t*)idx.p;
-            int64_t from = c->epoch;
-            while (from > col.ep[k]) {
-                WsComposeParams P;
-                memset(&P, 0, sizeof(P));
-                P.n = n_idx;
-                P.n_rows = c->n;
-                while (from > col.ep[k] && P.n_chain < WS_COMPOSE_MAX_CHAIN) {
-                    const int32_t* a = anc_of_event(c, from);
-                    if (a == nullptr) return fail(c, WS_EINVAL, "genealogy: ancestors of event %lld were released", (long long)from);
-                    P.chain[P.n_chain++] = a;
-                    --from;
-                }
-                CK(c, ws_launch_compose_rows(P, (int64_t*)rows.p, start, c->stream));
-                c->stats.kernel_launches++;
-                start = (const int64_t*)rows.p;
-            }
-            use = (const int64_t*)rows.p;
-        }
-        CK(c, ws_launch_gather_rows(col.front[k], use, n_idx, (double*)out.p, c->stream));
-        c->stats.kernel_launches++;
+        TRY(gather_rows_traced(c, col, k, (const int64_t*)idx.p, n_idx, rows, (double*)out.p));
         CK(c, cudaMemcpyAsync(host_out + (size_t)k * n_idx, out.p, sizeof(double) * (size_t)n_idx, cudaMemcpyDeviceToHost, c->stream));
     }
     CK(c, cudaStreamSynchronize(c->stream));
     return WS_OK;
 }
 
-// sample(state, n; replace) (src/utils.jl:102-118): n indices drawn with probability exp_norm(weights).  An analysis
-// call, not the hot path: the normalised weights are downloaded once and the draw is made on the host — with
-// replacement by inverting the sequential CDF at n Philox uniforms, without replacement by the Efraimidis-Spirakis
-// exponential-key selection.  Single-GPU states only: on a sharded state the indices would have to name (rank, row)
-// pairs of the GLOBAL posterior, which this interface cannot express, so the call is rejected instead of silently
-// sampling the local shard.
+// cross-rank hooks of a sharded describe / sample (ws_stats.h: WsStatsComm)
+static int stats_allgather_words(void* ctx, const unsigned long long* in, size_t words, unsigned long long* out);
+static int stats_allreduce_doubles(void* ctx, double* v, int n);
+static int stats_allreduce_u64_device(void* ctx, unsigned long long* d, size_t n);
+
+// Rows of GLOBAL particle indices.  Every rank reads the rows it owns into a zeroed n_idx x width buffer of bit patterns;
+// on a sharded state the buffers are summed as 64-bit integers, which is exact (one rank contributes each row) and
+// keeps -0.0 and NaN payloads.
+extern "C" int ws_col_download_global_rows(ws_ctx* c, int32_t id, const int64_t* global_indices, int64_t n_idx, double* host_out) {
+    if (!c || !global_indices || !host_out || n_idx <= 0)
+        return c ? fail(c, WS_EINVAL, "ws_col_download_global_rows: bad arguments") : WS_EINVAL;
+    if (id < 0 || id >= (int32_t)c->cols.size()) return fail(c, WS_EINVAL, "unknown column id %d", id);
+    for (int64_t i = 0; i < n_idx; ++i)
+        if (global_indices[i] < 0 || global_indices[i] >= c->n_global)
+            return fail(c, WS_EINVAL, "particle index %lld out of range", (long long)global_indices[i]);
+    TRY(flush_window(c));
+    const Column& col = c->cols[id];
+    if (c->nranks > 1) {  // sharded states have no genealogy: bring the planes into the current particle order first
+        std::vector<Plane> pl;
+        for (int k = 0; k < col.width; ++k) pl.push_back(Plane{id, k});
+        TRY(materialize_planes(c, &pl));
+    }
+    CK(c, cudaSetDevice(c->device));
+    std::vector<int64_t> loc, pos;  // local row and place in the output of the rows this rank owns
+    for (int64_t i = 0; i < n_idx; ++i) {
+        const int64_t r = global_indices[i] - c->offset;
+        if (r >= 0 && r < c->n) {
+            loc.push_back(r);
+            pos.push_back(i);
+        }
+    }
+    const int64_t n_own = (int64_t)loc.size();
+    const size_t total = (size_t)n_idx * (size_t)col.width;
+    TempBuf d_loc, d_pos, tmp, out, rows;
+    CK(c, cudaMalloc(&out.p, sizeof(double) * total));
+    CK(c, cudaMemsetAsync(out.p, 0, sizeof(double) * total, c->stream));
+    if (n_own > 0) {
+        CK(c, cudaMalloc(&d_loc.p, sizeof(int64_t) * (size_t)n_own));
+        CK(c, cudaMalloc(&d_pos.p, sizeof(int64_t) * (size_t)n_own));
+        CK(c, cudaMalloc(&tmp.p, sizeof(double) * (size_t)n_own));
+        CK(c, cudaMemcpyAsync(d_loc.p, loc.data(), sizeof(int64_t) * (size_t)n_own, cudaMemcpyHostToDevice, c->stream));
+        CK(c, cudaMemcpyAsync(d_pos.p, pos.data(), sizeof(int64_t) * (size_t)n_own, cudaMemcpyHostToDevice, c->stream));
+        c->stats.h2d_bytes += (int64_t)(2 * sizeof(int64_t)) * n_own;
+        for (int k = 0; k < col.width; ++k) {
+            TRY(gather_rows_traced(c, col, k, (const int64_t*)d_loc.p, n_own, rows, (double*)tmp.p));
+            CK(c, ws_sample_scatter_rows((const double*)tmp.p, (const int64_t*)d_pos.p, n_own, (double*)out.p + (size_t)k * n_idx, c->stream));
+            c->stats.kernel_launches++;
+        }
+    }
+    if (c->nranks > 1) TRY(stats_allreduce_u64_device(c, (unsigned long long*)out.p, total));
+    CK(c, cudaMemcpyAsync(host_out, out.p, sizeof(double) * total, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    c->stats.d2h_bytes += (int64_t)(sizeof(double) * total);
+    return WS_OK;
+}
+
+// sample(state, n; replace) (src/utils.jl:102-118): the draw include/wsb200.h defines, made on the device
+// (csrc/ws_kernels_stats.cu).  Nothing of size N leaves the device: only the n indices (and, without replacement, their
+// keys) come to the host.  Collective on a sharded state.
 extern "C" int ws_sample_indices(ws_ctx* c, int64_t n_draws, int replace, int64_t* indices_out) {
     if (!c || !indices_out) return WS_EINVAL;
     if (n_draws <= 0) return fail(c, WS_EINVAL, "Number of samples must be positive");
-    if (c->nranks > 1)
-        return fail(c, WS_EUNSUPPORTED, "sample(state, n) on a sharded state: local row indices cannot describe a draw from the global "
-                                        "posterior (use ws_expectation / ws_describe, or download the shards)");
-    if (!replace && n_draws > c->n) return fail(c, WS_EINVAL, "Cannot sample %lld particles without replacement from %lld particles", (long long)n_draws, (long long)c->n);
-    std::vector<double> w((size_t)c->n);
-    TRY(ws_exp_norm(c, w.data()));
+    if (!replace && n_draws > c->n_global)
+        return fail(c, WS_EINVAL, "Cannot sample %lld particles without replacement from %lld particles", (long long)n_draws, (long long)c->n_global);
+    TRY(ensure_reduced(c));  // flushes the window; m is the global maximum on a sharded state
+    const double m = c->h_red->m;
+    if (!std::isfinite(m)) return fail(c, WS_ENUMERIC, "sample(state, n): the largest log-weight is %g, so the weights cannot be normalised", m);
+    CK(c, cudaSetDevice(c->device));
     const uint64_t stream_id = c->next_stream++;
-    if (replace) {
-        std::vector<double> u((size_t)n_draws);
-        for (int64_t i = 0; i < n_draws; ++i) {
-            ws_u32x4 r = ws_philox4x32_10((uint64_t)i, stream_id, c->seed);
-            u[(size_t)i] = ws_u01(r.x, r.y);
-        }
-        std::vector<double> cdf((size_t)c->n);
-        double s = 0.0;
-        for (int64_t i = 0; i < c->n; ++i) {
-            s += w[(size_t)i];
-            cdf[(size_t)i] = s;
-        }
-        for (int64_t i = 0; i < n_draws; ++i) {
-            const double target = u[(size_t)i] * s;
-            int64_t idx = (int64_t)(std::lower_bound(cdf.begin(), cdf.end(), target) - cdf.begin());
-            if (idx >= c->n) idx = c->n - 1;
-            indices_out[i] = idx;
-        }
-    } else {
-        std::vector<std::pair<double, int64_t>> keys((size_t)c->n);
-        for (int64_t i = 0; i < c->n; ++i) {
-            ws_u32x4 r = ws_philox4x32_10((uint64_t)i, stream_id, c->seed);
-            const double e = -log(ws_u01_open0(r.x, r.y));
-            keys[(size_t)i] = {w[(size_t)i] > 0.0 ? e / w[(size_t)i] : INFINITY, i};
-        }
-        std::partial_sort(keys.begin(), keys.begin() + n_draws, keys.end());
-        for (int64_t i = 0; i < n_draws; ++i) indices_out[i] = keys[(size_t)i].second;
-    }
+    TRY(ensure_scratch(c, ws_sample_scratch_bytes(c->n, n_draws, replace)));
+    WsStatsComm comm{c, c->nranks, stats_allgather_words, stats_allreduce_doubles, stats_allreduce_u64_device, c->rank};
+    int launches = 0;
+    const cudaError_t e = ws_sample_draw(c->logw, c->n, c->offset, c->n_global, m, c->seed, stream_id, n_draws, replace, c->d_scratch,
+                                         c->stream, indices_out, &launches, &c->stats.d2h_bytes, c->nranks > 1 ? &comm : nullptr);
+    c->stats.kernel_launches += launches;
+    if (e == cudaErrorInvalidValue) return fail(c, WS_EINVAL, "sample(state, n): the draw is inconsistent across the ranks");
+    CK(c, e);
     return WS_OK;
 }
 
@@ -3897,7 +3936,6 @@ extern "C" int ws_set_lazy_gather(ws_ctx* c, int on) {
     c->lazy_gather = on != 0;
     return WS_OK;
 }
-// cross-rank hooks of a sharded describe (ws_stats.h: WsStatsComm)
 static int stats_allgather_words(void* ctx, const unsigned long long* in, size_t words, unsigned long long* out) {
     ws_ctx* c = (ws_ctx*)ctx;
     const size_t R = (size_t)c->nranks;
@@ -3928,7 +3966,7 @@ extern "C" int ws_describe(ws_ctx* c, int32_t n_planes, const int32_t* col, cons
     if (!c || !col || !comp || !out || n_planes < 1) return c ? fail(c, WS_EINVAL, "ws_describe: bad arguments") : WS_EINVAL;
     for (int t = 0; t < n_planes; ++t) TRY(check_plane(c, col[t], comp[t]));
     TRY(ensure_reduced(c));  // flushes the window; (m, S, Q) of the current log-weights (global on a sharded state)
-    WsStatsComm comm{c, c->nranks, stats_allgather_words, stats_allreduce_doubles, stats_allreduce_u64_device};
+    WsStatsComm comm{c, c->nranks, stats_allgather_words, stats_allreduce_doubles, stats_allreduce_u64_device, c->rank};
     if (c->nranks > 1) {  // sharded states have no genealogy: bring the planes into the current particle order first
         std::vector<Plane> pl;
         for (int t = 0; t < n_planes; ++t) pl.push_back(Plane{col[t], comp[t]});
