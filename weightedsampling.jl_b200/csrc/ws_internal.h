@@ -139,10 +139,9 @@ struct WsComposeParams {
 // launchers (ws_kernels.cu)
 cudaError_t ws_launch_vm(const WsVmProgram& P, int grid, cudaStream_t s);
 cudaError_t ws_launch_reduce_logw(const double* logw, int64_t n, WsLse* partials, int grid, cudaStream_t s);
-cudaError_t ws_launch_finalize(const WsLse* partials, int n_partials, int64_t n_global, double ess_perc_min,
-                               WsReduceOut* out, cudaStream_t s, unsigned long long* ties = nullptr);
-cudaError_t ws_launch_finalize_multi(const WsLse* partials, int n_partials, int k, int64_t n_global, double ess_perc_min, WsReduceOut* out,
-                                     cudaStream_t s);
+// k reductions of n_partials partials each (partials[j * n_partials ..] -> out[j]); ties: knife-edge decisions, or nullptr
+cudaError_t ws_launch_finalize(const WsLse* partials, int n_partials, int k, int64_t n_global, double ess_perc_min,
+                               WsReduceOut* out, unsigned long long* ties, cudaStream_t s);
 #define WS_SMALL_N 4096   // up to this many particles (single-GPU, Philox stratified / systematic) a Resample step is one kernel
                           // (one CTA: its time grows with N — 75 us at N = 1e4 against 45 us for the four launches of the tiled form)
 cudaError_t ws_launch_resample_small(const WsScanParams& P, const WsLse* partials, int n_partials, double ess_perc_min, WsReduceOut* out,

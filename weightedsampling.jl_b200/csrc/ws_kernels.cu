@@ -105,6 +105,52 @@ __device__ __forceinline__ WsLse lse_block_reduce(WsLse v, WsLse* warp_scratch /
     return v;
 }
 
+// (m, S, Q) of n_partials partials, combined in a fixed order; result valid in thread 0.
+template <int BLOCK>
+__device__ __forceinline__ WsLse lse_block_combine(const WsLse* __restrict__ partials, int n_partials, WsLse* warp_scratch /* BLOCK/32 */) {
+    WsLse part;
+    part.m = -INFINITY;
+    part.S = 0.0;
+    part.Q = 0.0;
+    for (int i = threadIdx.x; i < n_partials; i += BLOCK) part = lse_combine(part, partials[i]);
+    return lse_block_reduce<BLOCK>(part, warp_scratch);
+}
+
+// Sharded state: the ranks' (m, S, Q) triples (msq[3 r ..]) combined in rank order.  Every rank runs this on identical
+// inputs in identical order, so the ESS decision and the normalisation constants are bit-identical on all ranks.
+__device__ __forceinline__ WsLse lse_combine_ranks(const double* msq, int n_ranks) {
+    WsLse tot;
+    tot.m = -INFINITY;
+    tot.S = 0.0;
+    tot.Q = 0.0;
+    for (int r = 0; r < n_ranks; ++r) {
+        WsLse v;
+        v.m = msq[3 * r + 0];
+        v.S = msq[3 * r + 1];
+        v.Q = msq[3 * r + 2];
+        tot = lse_combine(tot, v);
+    }
+    return tot;
+}
+
+// The Resample decision (transformers.jl:474-498) from the combined (m, S, Q) of all n_global particles.
+// ESS% == ess_perc_min to within a few ulp: the reference's 1 / (N sum w^2) and this S^2 / (N Q) round differently
+// there (for exactly equal weights and ess_perc_min = 1.0 the reference fires for some N and not for others), so the
+// decision of such a step is rounding noise on both sides; they are counted into *ties (ws_get_ess_ties) when it is set.
+__device__ __forceinline__ void ws_decide(const WsLse& tot, int64_t n_global, double ess_perc_min, WsReduceOut* out,
+                                          unsigned long long* ties) {
+    out->m = tot.m;
+    out->S = tot.S;
+    out->Q = tot.Q;
+    const double lse = tot.m + log(tot.S);
+    out->lse = lse;
+    const double nn = (double)n_global;
+    out->ess_perc = (tot.S * tot.S) / (nn * tot.Q);  // 1 / (N * sum w^2), w = e / S
+    out->log_mean_w = lse - log(nn);
+    out->do_resample = (out->ess_perc < ess_perc_min) ? 1 : 0;  // NaN compares false, as in Julia
+    if (ties != nullptr && fabs(out->ess_perc - ess_perc_min) <= 8.0 * 2.220446049250313e-16 * fabs(ess_perc_min)) atomicAdd(ties, 1ull);
+}
+
 // ------------------------------------------------------------------------------------------
 // Fused elementwise window
 // ------------------------------------------------------------------------------------------
@@ -698,100 +744,27 @@ cudaError_t ws_launch_reduce_logw(const double* logw, int64_t n, WsLse* partials
     return cudaGetLastError();
 }
 
-// One CTA; fixed combination order => the decision is deterministic for a given grid size.
-// ESS% == ess_perc_min to within a few ulp: the reference's 1 / (N sum w^2) and this S^2 / (N Q) round differently
-// there (for exactly equal weights and ess_perc_min = 1.0 the reference fires for some N and not for others), so the
-// decision of such a step is rounding noise on both sides; they are counted (ws_get_ess_ties).
-__device__ __forceinline__ void ws_count_ess_tie(double ess, double ess_min, unsigned long long* ties) {
-    if (ties != nullptr && fabs(ess - ess_min) <= 8.0 * 2.220446049250313e-16 * fabs(ess_min)) atomicAdd(ties, 1ull);
-}
+// CTA j combines partials[j * n_partials ..] into out[j]: one CTA for a Resample step, K for the checkpoints of a
+// speculative block.  Fixed combination order => the decision is deterministic for a given number of partials.
 __global__ void __launch_bounds__(256) ws_finalize_kernel(const WsLse* __restrict__ partials, int n_partials,
                                                           int64_t n_global, double ess_perc_min,
                                                           WsReduceOut* __restrict__ out, unsigned long long* ties) {
     __shared__ WsLse warp_scratch[8];
-    WsLse part;
-    part.m = -INFINITY;
-    part.S = 0.0;
-    part.Q = 0.0;
-    for (int i = threadIdx.x; i < n_partials; i += 256) part = lse_combine(part, partials[i]);
-    WsLse tot = lse_block_reduce<256>(part, warp_scratch);
-    if (threadIdx.x == 0) {
-        out->m = tot.m;
-        out->S = tot.S;
-        out->Q = tot.Q;
-        const double lse = tot.m + log(tot.S);
-        out->lse = lse;
-        const double nn = (double)n_global;
-        out->ess_perc = (tot.S * tot.S) / (nn * tot.Q);  // 1 / (N * sum w^2), w = e / S
-        out->log_mean_w = lse - log(nn);
-        out->do_resample = (out->ess_perc < ess_perc_min) ? 1 : 0;  // NaN compares false, as in Julia
-        ws_count_ess_tie(out->ess_perc, ess_perc_min, ties);
-    }
+    const WsLse tot = lse_block_combine<256>(partials + (size_t)blockIdx.x * n_partials, n_partials, warp_scratch);
+    if (threadIdx.x == 0) ws_decide(tot, n_global, ess_perc_min, out + blockIdx.x, ties);
 }
 
-// K reductions at once (the checkpoints of a speculative block): CTA j finalizes partials[j * n_partials ...] into out[j]
-__global__ void __launch_bounds__(256) ws_finalize_multi_kernel(const WsLse* __restrict__ partials, int n_partials, int64_t n_global,
-                                                                double ess_perc_min, WsReduceOut* __restrict__ out) {
-    __shared__ WsLse warp_scratch[8];
-    const WsLse* mine = partials + (size_t)blockIdx.x * n_partials;
-    WsLse part;
-    part.m = -INFINITY;
-    part.S = 0.0;
-    part.Q = 0.0;
-    for (int i = threadIdx.x; i < n_partials; i += 256) part = lse_combine(part, mine[i]);
-    WsLse tot = lse_block_reduce<256>(part, warp_scratch);
-    if (threadIdx.x == 0) {
-        WsReduceOut* o = out + blockIdx.x;
-        o->m = tot.m;
-        o->S = tot.S;
-        o->Q = tot.Q;
-        const double lse = tot.m + log(tot.S);
-        o->lse = lse;
-        const double nn = (double)n_global;
-        o->ess_perc = (tot.S * tot.S) / (nn * tot.Q);
-        o->log_mean_w = lse - log(nn);
-        o->do_resample = (o->ess_perc < ess_perc_min) ? 1 : 0;
-    }
-}
-cudaError_t ws_launch_finalize_multi(const WsLse* partials, int n_partials, int k, int64_t n_global, double ess_perc_min, WsReduceOut* out,
-                                     cudaStream_t s) {
-    ws_finalize_multi_kernel<<<k, 256, 0, s>>>(partials, n_partials, n_global, ess_perc_min, out);
+cudaError_t ws_launch_finalize(const WsLse* partials, int n_partials, int k, int64_t n_global, double ess_perc_min,
+                               WsReduceOut* out, unsigned long long* ties, cudaStream_t s) {
+    ws_finalize_kernel<<<k, 256, 0, s>>>(partials, n_partials, n_global, ess_perc_min, out, ties);
     return cudaGetLastError();
 }
 
-cudaError_t ws_launch_finalize(const WsLse* partials, int n_partials, int64_t n_global, double ess_perc_min,
-                               WsReduceOut* out, cudaStream_t s, unsigned long long* ties) {
-    ws_finalize_kernel<<<1, 256, 0, s>>>(partials, n_partials, n_global, ess_perc_min, out, ties);
-    return cudaGetLastError();
-}
-
-// Sharded state: combine the ranks' (m, S, Q) triples (allgathered, rank order) into the global
-// reduction.  Every rank runs this on identical inputs in identical order, so the ESS decision and the
-// normalisation constants are bit-identical on all ranks.
+// Sharded state: combine the ranks' (m, S, Q) triples (allgathered, rank order) into the global reduction.
 __global__ void ws_finalize_global_kernel(const double* __restrict__ all_msq, int n_ranks, int64_t n_global,
                                           double ess_perc_min, WsReduceOut* __restrict__ out, unsigned long long* ties) {
     if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    WsLse tot;
-    tot.m = -INFINITY;
-    tot.S = 0.0;
-    tot.Q = 0.0;
-    for (int r = 0; r < n_ranks; ++r) {
-        WsLse v;
-        v.m = all_msq[3 * r + 0];
-        v.S = all_msq[3 * r + 1];
-        v.Q = all_msq[3 * r + 2];
-        tot = lse_combine(tot, v);
-    }
-    out->m = tot.m;
-    out->S = tot.S;
-    out->Q = tot.Q;
-    const double lse = tot.m + log(tot.S);
-    out->lse = lse;
-    const double nn = (double)n_global;
-    out->ess_perc = (tot.S * tot.S) / (nn * tot.Q);
-    out->log_mean_w = lse - log(nn);
-    out->do_resample = (out->ess_perc < ess_perc_min) ? 1 : 0;
-    ws_count_ess_tie(out->ess_perc, ess_perc_min, ties);
+    ws_decide(lse_combine_ranks(all_msq, n_ranks), n_global, ess_perc_min, out, ties);
 }
 
 cudaError_t ws_launch_finalize_global(const double* all_msq, int n_ranks, int64_t n_global, double ess_perc_min,
@@ -810,12 +783,7 @@ __global__ void __launch_bounds__(WS_MBOX_THREADS) ws_finalize_mbox_kernel(const
     __shared__ WsLse warp_scratch[WS_MBOX_THREADS / 32];
     __shared__ unsigned long long mine[3];
     __shared__ unsigned long long all[3 * WS_MBOX_MAX_RANKS];
-    WsLse part;
-    part.m = -INFINITY;
-    part.S = 0.0;
-    part.Q = 0.0;
-    for (int i = threadIdx.x; i < n_partials; i += WS_MBOX_THREADS) part = lse_combine(part, partials[i]);
-    const WsLse loc = lse_block_reduce<WS_MBOX_THREADS>(part, warp_scratch);
+    const WsLse loc = lse_block_combine<WS_MBOX_THREADS>(partials, n_partials, warp_scratch);
     if (threadIdx.x == 0) {
         mine[0] = (unsigned long long)__double_as_longlong(loc.m);
         mine[1] = (unsigned long long)__double_as_longlong(loc.S);
@@ -824,30 +792,9 @@ __global__ void __launch_bounds__(WS_MBOX_THREADS) ws_finalize_mbox_kernel(const
     __syncthreads();
     ws_mbox_allgather(M, M.seq, mine, 3, all);
     if (threadIdx.x != 0) return;
-    WsLse tot;
-    tot.m = -INFINITY;
-    tot.S = 0.0;
-    tot.Q = 0.0;
-    for (int r = 0; r < M.nranks; ++r) {
-        WsLse v;
-        v.m = __longlong_as_double((long long)all[3 * r + 0]);
-        v.S = __longlong_as_double((long long)all[3 * r + 1]);
-        v.Q = __longlong_as_double((long long)all[3 * r + 2]);
-        all_msq[3 * r + 0] = v.m;
-        all_msq[3 * r + 1] = v.S;
-        all_msq[3 * r + 2] = v.Q;
-        tot = lse_combine(tot, v);
-    }
-    out->m = tot.m;
-    out->S = tot.S;
-    out->Q = tot.Q;
-    const double lse = tot.m + log(tot.S);
-    out->lse = lse;
-    const double nn = (double)n_global;
-    out->ess_perc = (tot.S * tot.S) / (nn * tot.Q);
-    out->log_mean_w = lse - log(nn);
-    out->do_resample = (out->ess_perc < ess_perc_min) ? 1 : 0;
-    ws_count_ess_tie(out->ess_perc, ess_perc_min, ties);
+    const double* msq = reinterpret_cast<const double*>(all);   // the triples' bits, as they were sent
+    for (int k = 0; k < 3 * M.nranks; ++k) all_msq[k] = msq[k];
+    ws_decide(lse_combine_ranks(msq, M.nranks), n_global, ess_perc_min, out, ties);
 }
 cudaError_t ws_launch_finalize_mbox(const WsLse* partials, int n_partials, int64_t n_global, double ess_perc_min, WsReduceOut* out,
                                     double* all_msq, unsigned long long* ties, const WsMailbox& M, cudaStream_t s) {
@@ -2362,7 +2309,7 @@ __global__ void __maxnreg__(WS_CHAIN_MAXREG) ws_chain_kernel(const __grid_consta
 // ---- small particle sets: the whole Resample step in ONE kernel --------------------------------------------------
 // Below WS_SMALL_N particles a step is launch-latency bound: finalize, two memsets, tile CDF, offsets, search, heavy
 // expansion and the identity fill are eight stream operations of a few microseconds each.  One CTA does all of it:
-// the (m, S, Q) combination (the very code of ws_finalize_kernel: same order, same bits), the decision, the
+// the (m, S, Q) combination and the decision (those of ws_finalize_kernel: same order, same bits), the
 // fixed-point CDF in chunks with a running carry, F(C_m) per particle through the same ws_F_int, and the expansion by a
 // binary search of every slot in the F table.  Ancestors are bit-identical to the large-N kernels (integer sums).
 __global__ void __launch_bounds__(256) ws_resample_small_kernel(const __grid_constant__ WsScanParams P, const WsLse* __restrict__ partials,
@@ -2376,23 +2323,9 @@ __global__ void __launch_bounds__(256) ws_resample_small_kernel(const __grid_con
     (void)Ftab;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     if (do_finalize) {
-        WsLse part;
-        part.m = -INFINITY;
-        part.S = 0.0;
-        part.Q = 0.0;
-        for (int i = threadIdx.x; i < n_partials; i += 256) part = lse_combine(part, partials[i]);
-        WsLse tot = lse_block_reduce<256>(part, warp_scratch);
+        const WsLse tot = lse_block_combine<256>(partials, n_partials, warp_scratch);
         if (threadIdx.x == 0) {
-            out->m = tot.m;
-            out->S = tot.S;
-            out->Q = tot.Q;
-            const double lse = tot.m + log(tot.S);
-            out->lse = lse;
-            const double nn = (double)P.n_slots;
-            out->ess_perc = (tot.S * tot.S) / (nn * tot.Q);
-            out->log_mean_w = lse - log(nn);
-            out->do_resample = (out->ess_perc < ess_perc_min) ? 1 : 0;
-            ws_count_ess_tie(out->ess_perc, ess_perc_min, ties);
+            ws_decide(tot, P.n_slots, ess_perc_min, out, ties);
             __threadfence_block();
         }
         __syncthreads();

@@ -184,7 +184,6 @@ struct ws_ctx {
     int spec_pending = 0;
     bool logw_spec = false;
     bool async_resample = true;     // env WSB200_ASYNC_RESAMPLE=0: ws_resample_async behaves like ws_resample
-    bool merged_decision_wait = true;  // sharded steps: the decision is read with the slot bounds (env WSB200_MERGED_WAIT=0: two waits)
     bool small_resample = true;     // env WSB200_SMALL_RESAMPLE=0: small particle sets use the multi-kernel resampler too
     ws_resample_info last_info{};   // outcome of the most recent Resample step (ws_last_resample)
     bool last_info_pending = false; // ... which is the newest unresolved record
@@ -587,8 +586,6 @@ extern "C" int ws_create_sharded(ws_ctx** out, int64_t n_global, int rank, int n
     {
         const char* v = getenv("WSB200_ASYNC_RESAMPLE");
         c->async_resample = !(v != nullptr && strcmp(v, "0") == 0);
-        v = getenv("WSB200_MERGED_WAIT");
-        c->merged_decision_wait = !(v != nullptr && strcmp(v, "0") == 0);
         v = getenv("WSB200_SMALL_RESAMPLE");
         c->small_resample = !(v != nullptr && strcmp(v, "0") == 0);
     }
@@ -1404,7 +1401,8 @@ extern "C" int ws_sample_importance_normal(ws_ctx* c, int32_t col, int32_t comp,
 // reductions / resampling
 // ------------------------------------------------------------------------------------------
 // Bring the host's view up to date with the Resample steps it issued without looking at their outcome
-// (ws_resample_async): wait for the stream, read their records from the pinned ring in order.
+// (ws_resample_async): wait for the stream, read their records from the pinned ring in order.  Not book_step: these
+// steps were booked as fired when issued, and statements issued since may have changed the weights and the flags.
 static int resolve_spec(ws_ctx* c) {
     if (c->spec_pending == 0) return WS_OK;
     c->spec_immediate = (c->spec_pending == 1 && c->logw_spec) ? c->spec_immediate + 1 : 0;
@@ -1425,11 +1423,7 @@ static int resolve_spec(ws_ctx* c) {
     }
     c->spec_pending = 0;
     if (c->last_info_pending) {
-        c->last_info.fired = 1;
-        c->last_info.resampled = last.do_resample ? 1 : 0;
-        c->last_info.ess_perc = last.ess_perc;
-        c->last_info.log_mean_w = last.log_mean_w;
-        c->last_info.n_clamped = -1;
+        c->last_info = ws_resample_info{1, last.do_resample ? 1 : 0, last.ess_perc, last.log_mean_w, -1};
         c->last_info_pending = false;
     }
     if (c->logw_spec) {
@@ -1476,7 +1470,7 @@ static int ensure_reduced(ws_ctx* c, bool for_resample = false, bool wait = true
         timed_end(c, te);
     } else {
         timed_begin(c, KC_FINALIZE, te);
-        CK(c, ws_launch_finalize(c->d_partials, c->n_partials, c->n_global, c->ess_perc_min, c->d_red, c->stream, c->nranks > 1 ? nullptr : ties));
+        CK(c, ws_launch_finalize(c->d_partials, c->n_partials, 1, c->n_global, c->ess_perc_min, c->d_red, c->nranks > 1 ? nullptr : ties, c->stream));
         timed_end(c, te);
         if (c->nranks > 1) {
             // every rank reduces its shard; the (m, S, Q) triples are allgathered and combined in rank order
@@ -2505,6 +2499,22 @@ static int resample_sharded(ws_ctx* c, const double* d_ru, uint64_t stream_id, i
 
 static int spec_checkpoint(ws_ctx* c);
 
+// The outcome of a Resample step whose decision the host has read (transformers.jl:474-498).
+static void book_step(ws_ctx* c, const WsReduceOut& r, bool fired) {
+    if (fired) {
+        // fill!(state.weights, mean_logW): kept symbolic until somebody reads the array
+        c->logw_uniform = true;
+        c->logw_base = r.log_mean_w;
+        c->partials_valid = false;
+        c->red_valid = false;
+        c->stats.resamples_done++;
+    }
+    c->resampled = fired;
+    c->weights_changed = false;
+    c->last_info = ws_resample_info{1, fired ? 1 : 0, r.ess_perc, r.log_mean_w, -1};
+    c->last_info_pending = false;
+}
+
 extern "C" int ws_resample(ws_ctx* c, ws_resample_info* info) {
     if (!c) return WS_EINVAL;
     if (c->spec_block && !c->spec_flushing) return info ? fail(c, WS_EUNSUPPORTED, "ws_resample with an outcome inside a speculative block") : spec_checkpoint(c);
@@ -2523,48 +2533,21 @@ extern "C" int ws_resample(ws_ctx* c, ws_resample_info* info) {
     }
     if (c->resampler == WS_RESAMPLER_MULTINOMIAL && c->nranks > 1 && c->d_replay_u != nullptr)
         return fail(c, WS_EUNSUPPORTED, "multinomial resampling of a sharded state with replayed uniforms (Philox draws are supported)");
-    if (c->nranks > 1 && c->d_replay_u == nullptr && c->merged_decision_wait) {
-        // Sharded step: the decision travels with the slot bounds (one host wait per step instead of two).
-        TRY(ensure_reduced(c, true, /*wait=*/false));
-        c->stats.resamples_fired++;
-        const uint64_t step_stream = c->next_stream++;
-        int fired = 0;
-        if (c->red_valid) {   // (nothing was weighted on the device since the last reduction: *h_red is current)
-            fired = c->h_red->do_resample ? 1 : 0;
-            if (fired) {
-                TRY(begin_resample_event(c));
-                TRY(resample_sharded(c, nullptr, step_stream));
-            }
-        } else {
-            const auto tp0 = std::chrono::steady_clock::now();
-            TRY(prepare_resample_event(c));   // the half of begin_resample_event that moves planes (harmless if the step does not fire)
-            c->phase_ms[7] += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp0).count();
-            TRY(resample_sharded(c, nullptr, step_stream, &fired));
-        }
-        const WsReduceOut r = *c->h_red;
-        if (fired) {
-            c->logw_uniform = true;
-            c->logw_base = r.log_mean_w;
-            c->partials_valid = false;
-            c->red_valid = false;
-            c->resampled = true;
-            c->stats.resamples_done++;
-        } else {
-            c->resampled = false;
-        }
-        c->weights_changed = false;
-        c->last_info = ws_resample_info{1, fired, r.ess_perc, r.log_mean_w, -1};
-        c->last_info_pending = false;
-        if (info) *info = c->last_info;
-        return WS_OK;
-    }
-    TRY(ensure_reduced(c, true));
+    // Sharded step with Philox draws: the decision travels with the slot bounds (one host wait per step instead of two)
+    const bool merged = c->nranks > 1 && c->d_replay_u == nullptr;
+    TRY(ensure_reduced(c, true, /*wait=*/!merged));
     c->stats.resamples_fired++;
-    const WsReduceOut r = *c->h_red;
     // the Philox stream of this step's slot uniforms is taken whether or not the step fires, so that the streams of
     // everything that follows do not depend on how (or when) the decision is learnt
     const uint64_t step_stream = c->next_stream++;
-    if (r.do_resample) {
+    int fired = 0;
+    if (merged && !c->red_valid) {  // (*h_red is current when nothing was weighted on the device since the last reduction)
+        const auto tp0 = std::chrono::steady_clock::now();
+        TRY(prepare_resample_event(c));   // the half of begin_resample_event that moves planes (harmless if the step does not fire)
+        c->phase_ms[7] += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tp0).count();
+        TRY(resample_sharded(c, nullptr, step_stream, &fired));
+    } else if (c->h_red->do_resample) {
+        fired = 1;
         // slot uniforms: one per slot (stratified) or one in total (systematic), in replay order
         const double* d_ru = nullptr;
         if (c->d_replay_u != nullptr) {
@@ -2575,50 +2558,27 @@ extern "C" int ws_resample(ws_ctx* c, ws_resample_info* info) {
             d_ru = c->d_replay_u + c->cur_u;
             c->cur_u += need;
         }
-        if (c->nranks > 1) {
-            TRY(begin_resample_event(c));
-            TRY(resample_sharded(c, d_ru, step_stream));
-            c->logw_uniform = true;
-            c->logw_base = r.log_mean_w;
-            c->partials_valid = false;
-            c->red_valid = false;
-            c->resampled = true;
-            c->stats.resamples_done++;
-            c->weights_changed = false;
-            c->last_info = ws_resample_info{1, 1, r.ess_perc, r.log_mean_w, -1};
-            c->last_info_pending = false;
-            if (info) *info = c->last_info;
-            return WS_OK;
-        }
-        const uint64_t stream_id = step_stream;
         // planes still in an older order keep their ancestor vectors (genealogy) or are gathered now
         TRY(begin_resample_event(c));
-        const double* d_sorted = nullptr;
-        if (c->resampler == WS_RESAMPLER_MULTINOMIAL && d_ru != nullptr) {
-            TRY(sorted_replay_uniforms(c, d_ru, c->n, &d_sorted));   // replayed draws (tests): sorted on the host
-            d_ru = nullptr;
-        }
-        if (small_resample_ok(c, d_ru) && d_sorted == nullptr) {
-            TRY(run_small_resample(c, stream_id, 0, 0));
+        if (c->nranks > 1) {
+            TRY(resample_sharded(c, d_ru, step_stream));
         } else {
-            TRY(run_scan_search(c, c->logw, 0, c->resampler, c->n, d_ru, d_sorted, c->d_anc, c->d_tile_words, c->d_cdf_local, stream_id, c->d_counters + 0));
+            const double* d_sorted = nullptr;
+            if (c->resampler == WS_RESAMPLER_MULTINOMIAL && d_ru != nullptr) {
+                TRY(sorted_replay_uniforms(c, d_ru, c->n, &d_sorted));   // replayed draws (tests): sorted on the host
+                d_ru = nullptr;
+            }
+            if (small_resample_ok(c, d_ru) && d_sorted == nullptr) {
+                TRY(run_small_resample(c, step_stream, 0, 0));
+            } else {
+                TRY(run_scan_search(c, c->logw, 0, c->resampler, c->n, d_ru, d_sorted, c->d_anc, c->d_tile_words, c->d_cdf_local, step_stream, c->d_counters + 0));
+            }
+            // resample!(store, indices) is deferred: each plane is gathered when it is next read
+            end_resample_event(c);
+            if (!c->lazy_gather) TRY(materialize_planes(c));
         }
-        // resample!(store, indices) is deferred: each plane is gathered when it is next read
-        end_resample_event(c);
-        if (!c->lazy_gather) TRY(materialize_planes(c));
-        // fill!(state.weights, mean_logW): kept symbolic until somebody reads the array
-        c->logw_uniform = true;
-        c->logw_base = r.log_mean_w;
-        c->partials_valid = false;
-        c->red_valid = false;
-        c->resampled = true;
-        c->stats.resamples_done++;
-    } else {
-        c->resampled = false;
     }
-    c->weights_changed = false;
-    c->last_info = ws_resample_info{1, c->resampled ? 1 : 0, r.ess_perc, r.log_mean_w, -1};
-    c->last_info_pending = false;
+    book_step(c, *c->h_red, fired != 0);
     if (info) *info = c->last_info;
     return WS_OK;
 }
@@ -2633,17 +2593,12 @@ extern "C" int ws_resample(ws_ctx* c, ws_resample_info* info) {
 //     of the next pass reads through the ancestors either way, and that pass takes its old log-weights from
 //     d_red->log_mean_w or from the array according to the same flag (logw_mode 3).
 // `state.resampled`, the counters and anything that reads the log-weights resolve the pending records first
-// (resolve_spec), which is the only place the host waits.  Not taken (falls back to ws_resample): replayed
-// uniforms (the cursor advances only on a firing step), sharded states, multinomial, eager gather.
+// (resolve_spec), which is the only place the host waits.  Not taken (falls back to ws_resample): a step with nothing
+// to decide, replayed uniforms (the cursor advances only on a firing step), sharded states, multinomial, eager gather.
 extern "C" int ws_resample_async(ws_ctx* c) {
     if (!c) return WS_EINVAL;
     if (c->spec_block && !c->spec_flushing) return spec_checkpoint(c);
-    if (!c->weights_changed) {
-        c->last_info = ws_resample_info{0, -1, NAN, NAN, -1};
-        c->last_info_pending = false;
-        return WS_OK;
-    }
-    if (!c->async_resample || c->d_replay_u != nullptr || c->nranks > 1 || c->resampler == WS_RESAMPLER_MULTINOMIAL ||
+    if (!c->weights_changed || !c->async_resample || c->d_replay_u != nullptr || c->nranks > 1 || c->resampler == WS_RESAMPLER_MULTINOMIAL ||
         !c->lazy_gather || c->cols.empty() || c->spec_immediate >= 2)
         return ws_resample(c, nullptr);
     TRY(flush_window(c));
@@ -2670,7 +2625,7 @@ extern "C" int ws_resample_async(ws_ctx* c) {
     } else {
         TimedEvent te;
         timed_begin(c, KC_FINALIZE, te);
-        CK(c, ws_launch_finalize(c->d_partials, c->n_partials, c->n_global, c->ess_perc_min, c->d_red, c->stream, c->d_counters + 3));
+        CK(c, ws_launch_finalize(c->d_partials, c->n_partials, 1, c->n_global, c->ess_perc_min, c->d_red, c->d_counters + 3, c->stream));
         timed_end(c, te);
         CK(c, cudaMemcpyAsync(&c->h_ring[c->spec_head % ws_ctx::SPEC_RING], c->d_red, sizeof(WsReduceOut), cudaMemcpyDeviceToHost, c->stream));
         c->ring_event[c->spec_head % ws_ctx::SPEC_RING] = c->epoch + 1;
@@ -2860,7 +2815,7 @@ extern "C" int ws_exec_spec(ws_ctx* c, const ws_cmd* cmds, int32_t n_cmds, const
     if (rc != WS_OK) return rc;
     std::swap(c->logw, c->d_logw_bak);   // the pass wrote the other array: c->logw = after the block, d_logw_bak = before it
     const int grid = c->n_partials;
-    CK(c, ws_launch_finalize_multi(c->d_ck_partials, grid, K, c->n_global, c->ess_perc_min, c->d_ck_red, c->stream));
+    CK(c, ws_launch_finalize(c->d_ck_partials, grid, K, c->n_global, c->ess_perc_min, c->d_ck_red, nullptr, c->stream));
     CK(c, cudaMemcpyAsync(c->h_ck_red, c->d_ck_red, sizeof(WsReduceOut) * (size_t)K, cudaMemcpyDeviceToHost, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
     c->stats.kernel_launches += 1;
@@ -2874,14 +2829,12 @@ extern "C" int ws_exec_spec(ws_ctx* c, const ws_cmd* cmds, int32_t n_cmds, const
     if (first == K) {
         // nothing fired: the block is done
         const WsReduceOut& last = c->h_ck_red[K - 1];
+        // unlike a step of ws_resample, the block's last checkpoint is the reduction of the log-weights it leaves
         *c->h_red = last;
         CK(c, cudaMemcpyAsync(c->d_red, c->d_ck_red + (K - 1), sizeof(WsReduceOut), cudaMemcpyDeviceToDevice, c->stream));
         c->red_valid = true;
-        c->resampled = false;
-        c->weights_changed = false;
         c->stats.resamples_fired += K;
-        c->last_info = ws_resample_info{1, 0, last.ess_perc, last.log_mean_w, -1};
-        c->last_info_pending = false;
+        book_step(c, last, false);
         c->spec_steps.clear();
         *n_done = K;
         *fired = 0;
@@ -2993,7 +2946,7 @@ static int reduce_host_array(ws_ctx* c, const double* d_logw, int64_t n) {
     CK(c, ws_launch_reduce_logw(d_logw, n, c->d_partials, grid, c->stream));
     timed_end(c, te);
     timed_begin(c, KC_FINALIZE, te);
-    CK(c, ws_launch_finalize(c->d_partials, grid, n, c->ess_perc_min, c->d_red, c->stream));
+    CK(c, ws_launch_finalize(c->d_partials, grid, 1, n, c->ess_perc_min, c->d_red, nullptr, c->stream));
     timed_end(c, te);
     CK(c, cudaMemcpyAsync(c->h_red, c->d_red, sizeof(WsReduceOut), cudaMemcpyDeviceToHost, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
