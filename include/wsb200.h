@@ -100,7 +100,13 @@ enum ws_tok_op {
     WS_TOK_RANDPOISSON = 33,
     /* a constant supplied later: only inside the expressions of a ws_exec command list, where it is replaced by
      * params[col] before the statement is issued */
-    WS_TOK_PARAM = 34
+    WS_TOK_PARAM = 34,
+    /* build-time constant tables (ws_table below); `col` is the table id, the operands are popped:
+     * TABLE pops (row, column) and pushes T[row, column]; comp = 1 pushes log T[row, column] instead, with a column
+     * outside 1..n_cols giving -Inf without a fault (the log-probability of a Categorical value).
+     * RANDCAT pops the row and pushes a draw of Categorical(T[row, :]) (sampler expressions only). */
+    WS_TOK_TABLE = 35,
+    WS_TOK_RANDCAT = 36
 };
 
 typedef struct ws_tok {
@@ -116,6 +122,26 @@ typedef struct ws_expr {
     int32_t n;
     int32_t reserved;
 } ws_expr;
+
+/* ---- build-time constant tables ------------------------------------------------------------
+ * `vectorize` broadcasts `mu[s]` / `P[s, k]` like any getindex (src/rewrites.jl:146-219); here a Julia array that is a
+ * build-time constant and is indexed by a particle value becomes a table:
+ *   - A table is an n_rows x n_cols array of Float64, row-major; a vector is one row.  ws_table uploads it once per
+ *     context (deduplicated by content: the same values give the same id) and ws_destroy frees it.  Rows longer than
+ *     2^16 entries are WS_EUNSUPPORTED.
+ *   - Indices are Julia values, so 1-based: an index must be an integer-valued double in [1, n].  Any other index
+ *     (non-integer, out of range, NaN) gives NaN and never reads outside the table, and each such read adds one to
+ *     a sticky device counter of the context (ws_get_index_faults).  The reference throws BoundsError at the
+ *     statement; a host checks the counter when a run ends (DESIGN.md §7).
+ *   - Categorical(p), p a row of a table (a constant vector is a one-row table), with C_k = p_1 + ... + p_k summed
+ *     sequentially in Float64 on the host: the draw at one uniform u per particle (Philox, or the replayed uniform
+ *     stream, one per particle and draw in statement order, as for Uniform) is x = 1 + #{k < K : C_k <= u}:
+ *     Distributions 0.25's `while cp <= draw && i < n` walk over DiscreteNonParametric, found by a binary search.
+ *     logpdf(x) = log p_x for integer x in 1..K (log 0 = -Inf), -Inf for any other x.  Whether p is a probability
+ *     vector is the host's check (the Python front-end raises ValueError when the model is built).                */
+int ws_table(ws_ctx* ctx, const double* values, int64_t n_rows, int32_t n_cols, int32_t* id_out);
+/* out-of-range / non-integer / NaN table indices met so far by this context's kernels (flushes and waits) */
+int ws_get_index_faults(ws_ctx* ctx, int64_t* out);
 
 /* ---- lifecycle ---------------------------------------------------------------------------
  * SMCState(n; ess_perc_min = 0.5)  (src/types.jl:48-78): creates the device-resident state:

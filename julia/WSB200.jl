@@ -62,7 +62,7 @@ end
 const TOK_CONST, TOK_PLANE, TOK_ADD, TOK_SUB, TOK_MUL, TOK_DIV, TOK_NEG, TOK_EXP, TOK_LOG, TOK_SQRT, TOK_SQUARE,
       TOK_SIN, TOK_COS, TOK_ABS, TOK_POW, TOK_RANDN, TOK_RANDU, TOK_RANDEXP, TOK_LT, TOK_LE, TOK_EQ, TOK_SELECT,
       TOK_MIN, TOK_MAX, TOK_NOT, TOK_LGAMMA, TOK_LOG1P, TOK_EXPM1, TOK_TAN, TOK_ATAN, TOK_TANH, TOK_FLOOR,
-      TOK_RANDGAMMA, TOK_RANDPOISSON = Int32.(0:33)
+      TOK_RANDGAMMA, TOK_RANDPOISSON, TOK_PARAM, TOK_TABLE, TOK_RANDCAT = Int32.(0:36)
 
 function check(ctx, rc)
     rc == 0 && return nothing
@@ -325,6 +325,8 @@ const EXPR_KERNELS = IdDict{Any,Tuple{Function,Function}}(
     DK.Poisson => ((s, l) -> randpoisson_tok(tovec(s, l)), (l, x) -> ifelse(x >= 0.0, x * log(l) - l - loggamma_any(x + 1.0), -Inf)),
 )
 loggamma_any(a::DeviceVec) = loggamma(a)   # (every argument reaches these closures as a DeviceVec; constants are folded by the library)
+# Categorical and build-time arrays indexed by particle values (TOK_TABLE / TOK_RANDCAT over ws_table) are lowered by the
+# Python host only; this shim does not serialise such a getindex yet, so it keeps rejecting Categorical by name.
 const DEVICE_KERNEL_NAMES = Set{Symbol}([:Normal, :MvNormal, :Exponential, :Uniform, :LogNormal, :Bernoulli, :Laplace, :Cauchy,
                                         :Gamma, :Beta, :TDist, :Chisq, :InverseGamma, :Poisson])
 

@@ -8,7 +8,7 @@ types.  All particle work runs in ``lib/libwsb200.so`` (hand-written sm_100a CUD
 """
 from ._lib import LIB_PATH, UnsupportedModelError, WsError, load  # noqa: F401
 from .expr import (abs2, atan, col, cos, exp, expm1, floor, lgamma, log, log1p, maximum, minimum, randexp, randn,  # noqa: F401
-                   randu, sin, sqrt, tan, tanh, where)
+                   randu, sin, sqrt, table, tan, tanh, where)
 from .core import *  # noqa: F401,F403
 from .core import NormalDist  # noqa: F401
 from .analysis import (E, describe, ess_perc, exp_norm, expectation, icdf, log_evidence, logsumexp,  # noqa: F401

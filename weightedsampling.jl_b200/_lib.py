@@ -35,7 +35,7 @@ RESAMPLER = {"stratified": 0, "systematic": 1, "multinomial": 2}
 TOK_CONST, TOK_PLANE, TOK_ADD, TOK_SUB, TOK_MUL, TOK_DIV, TOK_NEG, TOK_EXP, TOK_LOG, TOK_SQRT, TOK_SQUARE, \
     TOK_SIN, TOK_COS, TOK_ABS, TOK_POW, TOK_RANDN, TOK_RANDU, TOK_RANDEXP, TOK_LT, TOK_LE, TOK_EQ, TOK_SELECT, TOK_MIN, \
     TOK_MAX, TOK_NOT, TOK_LGAMMA, TOK_LOG1P, TOK_EXPM1, TOK_TAN, TOK_ATAN, TOK_TANH, TOK_FLOOR, TOK_RANDGAMMA, \
-    TOK_RANDPOISSON, TOK_PARAM = range(35)
+    TOK_RANDPOISSON, TOK_PARAM, TOK_TABLE, TOK_RANDCAT = range(37)
 
 
 class ws_plane_stats(C.Structure):
@@ -152,6 +152,8 @@ SIGNATURES = {
     "ws_resample_host": (C.c_int, [_ctx, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, _i64p]),
     "ws_expectation": (C.c_int, [_ctx, _ep, C.c_int32, _dp]),
     "ws_sample_indices": (C.c_int, [_ctx, C.c_int64, C.c_int, C.c_void_p]),
+    "ws_table": (C.c_int, [_ctx, C.c_void_p, C.c_int64, C.c_int32, C.POINTER(C.c_int32)]),
+    "ws_get_index_faults": (C.c_int, [_ctx, _i64p]),
     "ws_col_download_rows": (C.c_int, [_ctx, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "ws_col_download_global_rows": (C.c_int, [_ctx, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]),
     "ws_move": (C.c_int, [_ctx, C.POINTER(ws_move_spec), C.POINTER(ws_move_info)]),

@@ -21,7 +21,7 @@ import numpy as np
 
 from . import _lib as L
 from ._lib import UnsupportedModelError, WsError, check
-from .expr import CExprs, Col, Const, Expr, Tokens, lower, wrap
+from .expr import CExprs, Col, Const, Expr, NotAProbabilityVector, Tokens, lower, wrap
 
 __all__ = [
     "DeviceColumnStore", "ColumnStore", "SMCState", "ParticleTransformer", "Assign", "AccessorAssign", "Sample",
@@ -82,6 +82,26 @@ class DeviceColumnStore:
         cid = C.c_int32()
         self._call("ws_col_ensure", name.encode(), int(width), C.byref(cid))
         return cid.value
+
+    def _table_id(self, tab):
+        """the context's id of a build-time table (uploaded on first use; ws_table deduplicates by content)"""
+        ids = self.__dict__.setdefault("_tables", {})
+        key = (tab.values.shape, tab.values.tobytes())
+        if key not in ids:
+            tid = C.c_int32()
+            self._call("ws_table", tab.values.ctypes.data_as(C.c_void_p), int(tab.values.shape[0]), int(tab.values.shape[1]),
+                       C.byref(tid))
+            ids[key] = tid.value
+        return ids[key]
+
+    def _new_index_faults(self):
+        """table index faults since the last call (0 without a call to the device when no table exists)"""
+        if not self.__dict__.get("_tables"):
+            return 0
+        n = C.c_int64()
+        self._call("ws_get_index_faults", C.byref(n))
+        new, self._faults_seen = n.value - self.__dict__.get("_faults_seen", 0), n.value
+        return new
 
     def close(self):
         if getattr(self, "_ctx", None) is not None and self._ctx:
@@ -371,7 +391,7 @@ class WeightedKernel:
     def _trace(self, fn, args, what):
         try:
             out = fn(*args)
-        except UnsupportedModelError:
+        except (UnsupportedModelError, NotAProbabilityVector):
             raise
         except Exception as e:  # e.g. math.exp(Expr), float(Expr)
             raise _unsupported(f"{self.name}.{what} is not a device expression ({type(e).__name__}: {e})")
@@ -579,6 +599,9 @@ def _expr_kernels():
     k["Chisq"] = WeightedKernel(lambda v: 2.0 * E.randgamma(v / 2.0), None,
                                 lambda v, x: E.where(x >= 0.0, (v / 2.0 - 1.0) * E.log(x) - x / 2.0 - E.lgamma(v / 2.0) - (v / 2.0) * LOG2,
                                                      NEG_INF), "Chisq")
+    # Categorical(p), p a constant probability vector or a row P[s, :] of a build-time matrix (expr.Table): the draw
+    # inverts the row's sequential partial sums at one uniform, the logpdf reads the row's logarithms (include/wsb200.h)
+    k["Categorical"] = WeightedKernel(lambda p: E.randcat(p), None, lambda p, x: E.cat_logpdf(p, x), "Categorical")
     k["InverseGamma"] = WeightedKernel(lambda a, t: t / E.randgamma(a), None,
                                        lambda a, t, x: E.where(x > 0.0, a * E.log(t) - E.lgamma(a) - (a + 1.0) * E.log(x) - t / x, NEG_INF),
                                        "InverseGamma")
@@ -755,6 +778,9 @@ class _Recorder:
 
     def _lookup(self, name):
         return self.store._lookup(name)
+
+    def _table_id(self, tab):
+        return self.store._table_id(tab)
 
     def _ensure(self, name, width):
         cid, w = self.store._lookup(name)
@@ -1200,6 +1226,10 @@ def run(root, state):
     state._root = root
     state._tape_valid = record
     root.apply(state)
+    faults = st._new_index_faults()
+    if faults:
+        raise IndexError(f"{faults} table reads had an index that is not an integer in range (Julia would throw a "
+                         "BoundsError); those values are NaN")
     return state
 
 

@@ -48,6 +48,49 @@ struct RngCursor {
     int64_t* variates = nullptr;  // replay cursor of the WS_OP_RANDV ops (accepted Gamma / Poisson variates)
 };
 
+// A build-time constant table as the lowering sees it (include/wsb200.h: ws_table): the addresses of its values, of
+// their logarithms and of its row-wise sequential partial sums, each array behind its own WsTableHdr.  Device
+// addresses in the runtime, host addresses in tests/host/.
+struct TableRef {
+    uint64_t values, logv, cdf;
+    int64_t n_rows;
+    int32_t n_cols;
+};
+
+// The memory image of a table (ws_table): three arrays, each [WsTableHdr | n_rows * n_cols doubles] — the values, their
+// logarithms, and the sequential Float64 partial sums of each row (cp += p[i], the order Distributions sums in).  The
+// runtime uploads it as it is; tests/host/ uses it in place.  TableRef addresses point at image + table_offset(k).
+inline size_t table_segment(int64_t n_rows, int32_t n_cols) { return 2 + (size_t)n_rows * (size_t)n_cols; }
+inline std::vector<double> table_image(const double* values, int64_t n_rows, int32_t n_cols) {
+    static_assert(sizeof(WsTableHdr) == 2 * sizeof(double), "a table header is two doubles");
+    const size_t seg = table_segment(n_rows, n_cols), ne = seg - 2;
+    std::vector<double> h(3 * seg, 0.0);
+    for (int k = 0; k < 3; ++k) {
+        const WsTableHdr hdr{0ull, n_rows};
+        memcpy(&h[k * seg], &hdr, sizeof hdr);
+    }
+    double* hv = &h[2];
+    double* hl = &h[seg + 2];
+    double* hc = &h[2 * seg + 2];
+    for (size_t i = 0; i < ne; ++i) {
+        hv[i] = values[i];
+        hl[i] = log(values[i]);
+    }
+    for (int64_t r = 0; r < n_rows; ++r) {
+        double cp = 0.0;
+        for (int32_t k = 0; k < n_cols; ++k) {
+            cp += values[(size_t)r * n_cols + k];
+            hc[(size_t)r * n_cols + k] = cp;
+        }
+    }
+    return h;
+}
+inline TableRef table_ref_at(const double* image, int64_t n_rows, int32_t n_cols) {
+    const size_t seg = table_segment(n_rows, n_cols);
+    return TableRef{(uint64_t)(uintptr_t)(image + 2), (uint64_t)(uintptr_t)(image + seg + 2), (uint64_t)(uintptr_t)(image + 2 * seg + 2),
+                    n_rows, n_cols};
+}
+
 // One fusion window (or the persistent score program): micro-ops + register allocation.
 struct Program {
     int max_regs = 64, max_ops = 96, max_io = 24;
@@ -75,6 +118,7 @@ struct Program {
     size_t stmt_begin_ops = 0;  // ops.size() when the current statement started
     int stmt_cache_ops = 0;     // sigma-cache prologue ops of the current statement (kept at its very start)
     RngCursor* rng = nullptr;  // set while a sampler expression is being lowered (WS_TOK_RAND*)
+    const std::vector<TableRef>* tables = nullptr;  // the context's tables, by id (WS_TOK_TABLE, WS_TOK_RANDCAT)
     int n_statements = 0;
     bool overflow = false;
     std::string error;
@@ -374,6 +418,39 @@ struct Program {
         return Val::lin(0.0, 1.0, t);
     }
 
+    // ---- tables ---------------------------------------------------------------------------------
+    const TableRef* table_ref(int32_t id) {
+        if (tables == nullptr || id < 0 || id >= (int32_t)tables->size()) {
+            fail("unknown table id");
+            return nullptr;
+        }
+        return &(*tables)[(size_t)id];
+    }
+    static double addr_bits(uint64_t addr) {
+        double b;
+        memcpy(&b, &addr, 8);
+        return b;
+    }
+    // T[row, col] (logp: log T[row, col] with a column outside 1..n_cols giving -Inf, the log-probability of a Categorical)
+    Val table_read(const TableRef& t, const Val& row, const Val& col, bool logp) {
+        const int ra = row.is_const ? (int)WS_REG_NONE : materialize(row);
+        const int rb = col.is_const ? (int)WS_REG_NONE : materialize(col);
+        const int d = alloc_temp();
+        emit(ws_make_op(WS_OP_TABLE, d, ra, rb, WS_REG_NONE, (uint32_t)t.n_cols | (logp ? WS_TABLE_LOGP : 0u),
+                        addr_bits(logp ? t.logv : t.values), row.is_const ? row.c0 : 0.0, col.is_const ? col.c0 : 0.0));
+        return Val::lin(0.0, 1.0, d);
+    }
+    // Categorical(T[row, :]): one uniform per particle (an ordinary WS_OP_RANDU: replay and Philox as for Uniform), then
+    // the search of that row's partial sums
+    Val categorical(const TableRef& t, const Val& row) {
+        const int rb = row.is_const ? (int)WS_REG_NONE : materialize(row);
+        const Val u = variate(WS_TOK_RANDU);
+        if (!error.empty()) return Val::constant(NAN);
+        const int d = alloc_temp();
+        emit(ws_make_op(WS_OP_CAT, d, u.reg, rb, WS_REG_NONE, (uint32_t)t.n_cols, addr_bits(t.cdf), row.is_const ? row.c0 : 0.0, 0.0));
+        return Val::lin(0.0, 1.0, d);
+    }
+
     // postfix tokens -> Val
     Val compile(const ws_expr& e) {
         std::vector<Val> st;
@@ -429,6 +506,30 @@ struct Program {
                     else if (t.op == WS_TOK_MAX) r = minmax(1, a, b);
                     else r = power(a, b);
                     st.push_back(r);
+                } break;
+                case WS_TOK_TABLE: {
+                    if (st.size() < 2) {
+                        fail("malformed expression (a table read needs a row and a column)");
+                        return Val::constant(NAN);
+                    }
+                    const TableRef* tr = table_ref(t.col);
+                    if (tr == nullptr) return Val::constant(NAN);
+                    Val cl = st.back();
+                    st.pop_back();
+                    Val rw = st.back();
+                    st.pop_back();
+                    st.push_back(table_read(*tr, rw, cl, t.comp == 1));
+                } break;
+                case WS_TOK_RANDCAT: {
+                    if (st.empty()) {
+                        fail("malformed expression (a Categorical draw needs its row)");
+                        return Val::constant(NAN);
+                    }
+                    const TableRef* tr = table_ref(t.col);
+                    if (tr == nullptr) return Val::constant(NAN);
+                    Val rw = st.back();
+                    st.pop_back();
+                    st.push_back(categorical(*tr, rw));
                 } break;
                 case WS_TOK_RANDGAMMA:
                 case WS_TOK_RANDPOISSON: {
@@ -508,7 +609,8 @@ struct Program {
             WsOp& last = ops.back();
             const uint32_t lop = last.w0 & 0xFFu;
             const uint32_t ldst = (last.w0 >> 8) & 0xFFu;
-            if ((int)ldst == v.reg && (lop <= WS_OP_POW || (lop >= WS_OP_CMP && lop <= WS_OP_MINMAX))) {
+            if ((int)ldst == v.reg && (lop <= WS_OP_POW || (lop >= WS_OP_CMP && lop <= WS_OP_MINMAX) || lop == WS_OP_TABLE ||
+                                       lop == WS_OP_CAT)) {
                 last.w0 = (last.w0 & ~0xFF00u) | ((uint32_t)dst << 8);
                 return;
             }

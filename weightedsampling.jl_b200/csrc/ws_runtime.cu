@@ -254,6 +254,12 @@ struct ws_ctx {
     int64_t n_tiles = 0;
     unsigned long long* d_counters = nullptr;  // [0] clamped slots (cumulative), [1] clamped (host-array calls), [2] MH accepts
 
+    // build-time constant tables (ws_table): one device allocation per table, [values | logs | partial sums], each
+    // array behind its WsTableHdr; `table_ids` finds a table by its content
+    std::vector<wsl::TableRef> tables;
+    std::vector<double*> table_mem;
+    std::map<std::string, int32_t> table_ids;
+
     // fusion window + score tape
     Program win;
     Program score;
@@ -336,6 +342,7 @@ static int map_for_epoch(ws_ctx* c, int64_t ep, const int32_t** out);
 static const int32_t* anc_of_event(const ws_ctx* c, int64_t event);
 static int materialize_tape_planes(ws_ctx* c, int32_t n_extra, const int32_t* col, const int32_t* comp);
 static int resolve_spec(ws_ctx* c);
+static int flush_window(ws_ctx* c);
 static int mbox_setup(ws_ctx* c);
 static WsMailbox mbox_next(ws_ctx* c, int n_exchanges);
 static int mbox_check(ws_ctx* c);
@@ -492,12 +499,14 @@ static int ensure_h_scratch(ws_ctx* c, size_t bytes) {
 // ------------------------------------------------------------------------------------------
 static void reset_window(ws_ctx* c) {
     c->win = Program();
+    c->win.tables = &c->tables;
     c->win.max_regs = WS_VM_MAX_REGS;
     c->win.max_ops = WS_VM_MAX_OPS;
     c->win.max_io = WS_VM_MAX_IO;
 }
 static void reset_score(ws_ctx* c) {
     c->score = Program();
+    c->score.tables = &c->tables;
     c->score.score_mode = true;
     c->score.temp_base = 0;
     c->score.n_temp_slots = WS_SCORE_TEMPS;
@@ -727,6 +736,7 @@ extern "C" int ws_destroy(ws_ctx* c) {
     if (c->d_mbox) cudaFree(c->d_mbox);
     if (c->h_mbox_err) cudaFreeHost(c->h_mbox_err);
     if (c->comm) g_nccl.CommDestroy(c->comm);
+    for (double* t : c->table_mem) cudaFree(t);
     cudaFree(c->d_score_ops);
     cudaFree(c->d_seg_ops);
     cudaFree(c->d_replay_n);
@@ -763,8 +773,63 @@ static int check_plane(ws_ctx* c, int32_t col, int32_t comp) {
 }
 static int check_expr(ws_ctx* c, const ws_expr* e, const char* what) {
     if (e == nullptr || e->toks == nullptr || e->n <= 0) return fail(c, WS_EINVAL, "%s: empty expression", what);
-    for (int i = 0; i < e->n; ++i)
-        if (e->toks[i].op == WS_TOK_PLANE) TRY(check_plane(c, e->toks[i].col, e->toks[i].comp));
+    for (int i = 0; i < e->n; ++i) {
+        const ws_tok& t = e->toks[i];
+        if (t.op == WS_TOK_PLANE) TRY(check_plane(c, t.col, t.comp));
+        if ((t.op == WS_TOK_TABLE || t.op == WS_TOK_RANDCAT) && (t.col < 0 || t.col >= (int32_t)c->tables.size()))
+            return fail(c, WS_EINVAL, "%s: unknown table id %d", what, t.col);
+        if (t.op == WS_TOK_TABLE && t.comp != 0 && t.comp != 1) return fail(c, WS_EINVAL, "%s: table read mode %d", what, t.comp);
+    }
+    return WS_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// build-time constant tables
+// ------------------------------------------------------------------------------------------
+extern "C" int ws_table(ws_ctx* c, const double* values, int64_t n_rows, int32_t n_cols, int32_t* id_out) {
+    if (!c || !values || !id_out) return WS_EINVAL;
+    if (n_rows < 1 || n_cols < 1) return fail(c, WS_EINVAL, "ws_table: a table needs a row and a column (got %lld x %d)", (long long)n_rows, n_cols);
+    if (n_cols > WS_TABLE_MAX_COLS)
+        return fail(c, WS_EUNSUPPORTED, "ws_table: rows of %d entries (at most %d are supported)", n_cols, WS_TABLE_MAX_COLS);
+    if (n_rows > ((int64_t)1 << 36) / n_cols) return fail(c, WS_EINVAL, "ws_table: %lld x %d entries is too large", (long long)n_rows, n_cols);
+    const size_t ne = (size_t)n_rows * (size_t)n_cols;
+    std::string key((const char*)&n_cols, sizeof n_cols);
+    key.append((const char*)values, sizeof(double) * ne);
+    auto it = c->table_ids.find(key);
+    if (it != c->table_ids.end()) {
+        *id_out = it->second;
+        return WS_OK;
+    }
+    const std::vector<double> h = wsl::table_image(values, n_rows, n_cols);
+    CK(c, cudaSetDevice(c->device));
+    double* d = nullptr;
+    CK(c, cudaMalloc(&d, sizeof(double) * h.size()));
+    c->table_mem.push_back(d);
+    CK(c, cudaMemcpyAsync(d, h.data(), sizeof(double) * h.size(), cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    c->stats.h2d_bytes += (int64_t)(sizeof(double) * h.size());
+    c->tables.push_back(wsl::table_ref_at(d, n_rows, n_cols));
+    *id_out = (int32_t)c->tables.size() - 1;
+    c->table_ids.emplace(std::move(key), *id_out);
+    return WS_OK;
+}
+
+extern "C" int ws_get_index_faults(ws_ctx* c, int64_t* out) {
+    if (!c || !out) return WS_EINVAL;
+    TRY(flush_window(c));
+    const size_t n = c->table_mem.size() * 3;
+    TRY(ensure_h_scratch(c, sizeof(WsTableHdr) * std::max<size_t>(1, n)));
+    WsTableHdr* hh = reinterpret_cast<WsTableHdr*>(c->h_scratch);
+    for (size_t t = 0; t < c->table_mem.size(); ++t) {
+        const size_t seg = wsl::table_segment(c->tables[t].n_rows, c->tables[t].n_cols);
+        for (int k = 0; k < 3; ++k)
+            CK(c, cudaMemcpyAsync(&hh[t * 3 + k], c->table_mem[t] + k * seg, sizeof(WsTableHdr), cudaMemcpyDeviceToHost, c->stream));
+    }
+    CK(c, cudaStreamSynchronize(c->stream));
+    int64_t s = 0;
+    for (size_t k = 0; k < n; ++k) s += (int64_t)hh[k].faults;
+    c->stats.d2h_bytes += (int64_t)(sizeof(WsTableHdr) * n);
+    *out = s;
     return WS_OK;
 }
 
@@ -939,6 +1004,7 @@ static int tape_statement(ws_ctx* c, std::function<void(Program&)> lower, std::v
             // too many distinct planes for one register file: from now on the tape is folded in segments
             c->score_wide = true;
             c->score = Program();
+            c->score.tables = &c->tables;
         }
     }
     const int32_t cache_ops = c->score_wide ? 0 : (int32_t)c->score.stmt_cache_ops;
@@ -2769,6 +2835,7 @@ extern "C" int ws_exec_spec(ws_ctx* c, const ws_cmd* cmds, int32_t n_cmds, const
         c->tape.resize(tape_size);
         if (c->score_wide != s_wide) {
             c->score = Program();   // the tape went wide inside the block: it is folded from its entries anyway
+            c->score.tables = &c->tables;
         } else if (!c->score_wide) {
             c->score.rollback(score_mark);
             c->d_score_uploaded = std::min(c->d_score_uploaded, c->score.ops.size());
@@ -3068,6 +3135,7 @@ extern "C" int ws_expectation(ws_ctx* c, const ws_expr* f, int32_t n_exprs, doub
     for (int k = 0; k < n_exprs; ++k) TRY(check_expr(c, &f[k], "ws_expectation"));
     TRY(ensure_reduced(c));
     Program p;
+    p.tables = &c->tables;
     p.max_regs = WS_VM_MAX_REGS;
     p.max_ops = WS_VM_MAX_OPS;
     p.max_io = WS_VM_MAX_IO;
@@ -3377,8 +3445,9 @@ static int for_each_tape_segment(ws_ctx* c, int64_t target_depth, const std::vec
         const int v = e ? atoi(e) : WS_SCORE_SEG_REGS;
         return std::min(WS_SCORE_MAX_REGS, std::max(WS_SCORE_TEMPS + 4, v));
     }();
-    auto fresh = [] {
+    auto fresh = [c] {
         Program p;
+        p.tables = &c->tables;
         p.score_mode = true;
         p.temp_base = 0;
         p.n_temp_slots = WS_SCORE_TEMPS;

@@ -41,6 +41,12 @@ enum WsOpCode : uint32_t {
     ,
     WS_OP_RANDV = 19  // r[dst] = variate with a parameter A = a==NONE ? k2 : r[a];  imm: 0 standard Gamma(shape A),
                       // 1 Poisson(A).  k0 = Philox stream; replay: r[dst] = replay_v[(int64)k1 + particle]
+    ,
+    WS_OP_TABLE = 20  // r[dst] = T[(ROW-1)*n_cols + (COL-1)]   ROW = a==NONE ? k1 : r[a];  COL = b==NONE ? k2 : r[b];
+                      // k0 = the table's device address (bit-cast), imm = n_cols | WS_TABLE_LOGP (see ws_table_read)
+    ,
+    WS_OP_CAT = 21  // r[dst] = 1 + #{k < K : C[(ROW-1)*K + k-1] <= U}   U = r[a];  ROW = b==NONE ? k1 : r[b];
+                    // k0 = the address of the table's row-wise partial sums C (bit-cast), imm = K (ws_cat_draw)
 };
 
 enum WsUnary : uint32_t {
@@ -106,6 +112,56 @@ WS_HD uint64_t ws_double_bits(double v) {
     memcpy(&b, &v, 8);
     return b;
 #endif
+}
+
+// ---- build-time constant tables (WS_OP_TABLE, WS_OP_CAT; include/wsb200.h: ws_table) ------------------------------
+// A device table is [WsTableHdr | n_rows * n_cols doubles, row-major]; the ops carry the address of the data, so the
+// header is found just below it.  Indices are Julia's: 1-based integer-valued doubles.  Any other index (non-integer,
+// out of range, NaN) reads nothing, gives NaN and counts one fault in the header (ws_get_index_faults sums them).
+struct alignas(16) WsTableHdr {
+    unsigned long long faults;
+    int64_t n_rows;
+};
+#define WS_TABLE_MAX_COLS 65536
+#define WS_TABLE_COLS_MASK 0x1FFFFu
+// the column is the value of a Categorical: outside 1..n_cols it is outside the support, log-probability -Inf, no fault
+#define WS_TABLE_LOGP (1u << 23)
+
+WS_HD const double* ws_table_ptr(double k0) { return reinterpret_cast<const double*>((uintptr_t)ws_double_bits(k0)); }
+WS_HD void ws_table_fault(const double* T) {
+    unsigned long long* f = &(reinterpret_cast<WsTableHdr*>(const_cast<double*>(T)) - 1)->faults;
+#if defined(__CUDA_ARCH__)
+    atomicAdd(f, 1ull);
+#else
+    ++*f;
+#endif
+}
+WS_HD bool ws_table_index_ok(double x, int64_t n) { return x >= 1.0 && x <= (double)n && x == floor(x); }
+WS_HD double ws_table_read(const double* T, uint32_t imm, double row, double col) {
+    const int64_t n_cols = (int64_t)(imm & WS_TABLE_COLS_MASK);
+    const int64_t n_rows = (reinterpret_cast<const WsTableHdr*>(T) - 1)->n_rows;
+    const bool row_ok = ws_table_index_ok(row, n_rows);
+    if (row_ok && ws_table_index_ok(col, n_cols)) return T[((int64_t)row - 1) * n_cols + ((int64_t)col - 1)];
+    if (row_ok && (imm & WS_TABLE_LOGP)) return -INFINITY;
+    ws_table_fault(T);
+    return NAN;
+}
+// Categorical(C's row) at uniform u: Distributions' `while cp <= u && i < K` walk over the sequential partial sums,
+// i.e. 1 + the number of C_1 .. C_{K-1} that are <= u, found by a binary search (C is non-decreasing)
+WS_HD double ws_cat_draw(const double* C, uint32_t K, double row, double u) {
+    const int64_t n_rows = (reinterpret_cast<const WsTableHdr*>(C) - 1)->n_rows;
+    if (!ws_table_index_ok(row, n_rows)) {
+        ws_table_fault(C);
+        return NAN;
+    }
+    const double* c = C + ((int64_t)row - 1) * (int64_t)K;
+    uint32_t lo = 0, hi = K - 1;  // count of c[0 .. K-2] that are <= u lies in [lo, hi]
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (c[mid] <= u) lo = mid + 1;
+        else hi = mid;
+    }
+    return (double)(lo + 1);
 }
 
 // Decoded micro-op: what the interpreter executes.  The 32-byte WsOp is what the lowering emits and what
@@ -307,6 +363,23 @@ WS_HD void ws_vm_exec_d(const WsDop& o, double* __restrict__ R, double (&acc)[P]
                                     : ws_rand_poisson(A, particle[j], ws_double_bits(k0), rng.seed);
                 }
                 Rd[j * STRIDE] = v;
+            }
+        } break;
+        case WS_OP_TABLE: {
+            const double* T = ws_table_ptr(k0);
+#pragma unroll
+            for (int j = 0; j < P; ++j) {
+                const double row = (a == WS_OFF_NONE) ? k1 : Ra[j * STRIDE];
+                const double col = (b == WS_OFF_NONE) ? k2 : Rb[j * STRIDE];
+                Rd[j * STRIDE] = ws_table_read(T, imm, row, col);
+            }
+        } break;
+        case WS_OP_CAT: {
+            const double* Ct = ws_table_ptr(k0);
+#pragma unroll
+            for (int j = 0; j < P; ++j) {
+                const double row = (b == WS_OFF_NONE) ? k1 : Rb[j * STRIDE];
+                Rd[j * STRIDE] = ws_cat_draw(Ct, imm, row, Ra[j * STRIDE]);
             }
         } break;
         case WS_OP_LOGPDF_NORMAL: {

@@ -145,6 +145,17 @@ inline void ws_sl_canonical(const Prog& P, uint8_t (&map)[256]) {
     }
 }
 
+// Table reads and Categorical draws (WS_OP_TABLE, WS_OP_CAT) dereference a table address and may count index faults:
+// no signature has them, and a window that contains one always runs on the interpreter
+template <class Prog>
+inline bool ws_sl_has_table_ops(const Prog& P, int n_ops) {
+    for (int i = 0; i < n_ops; ++i) {
+        const uint32_t op = P.ops[i].w0 & 0xFFu;
+        if (op == WS_OP_TABLE || op == WS_OP_CAT) return true;
+    }
+    return false;
+}
+
 template <class Sig, class Prog>
 inline bool ws_sl_matches(const Prog& P, const uint8_t (&map)[256]) {
     if (P.n_expect != 0 || P.n_ops != Sig::n_ops || P.n_loads != Sig::n_loads || P.n_stores != Sig::n_stores) return false;
@@ -180,6 +191,7 @@ inline bool ws_sl_matches_repeated(const Prog& P, int max_reps) {
     };
     const int r = P.n_ckpt;
     if (r < 1 || r > max_reps || Sig::n_stores != 0 || P.n_stores != 0 || P.n_ops != r * Sig::n_ops) return false;
+    if (ws_sl_has_table_ops(P, P.n_ops)) return false;
     for (int j = 0; j < r; ++j)
         if ((int)P.ckpt_pc[j] != (j + 1) * Sig::n_ops - 1) return false;
     View v{Sig::n_ops, P.n_loads, 0, P.n_expect, P.load_reg, P.store_reg, P.ops};
@@ -194,6 +206,7 @@ inline bool ws_sl_matches_repeated(const Prog& P, int max_reps) {
 
 template <class Prog>
 inline int ws_sl_find(const Prog& P) {
+    if (ws_sl_has_table_ops(P, P.n_ops)) return -1;
     uint8_t map[256];
     ws_sl_canonical(P, map);
 #define WS_SL_TRY(idx, Sig) \

@@ -125,6 +125,108 @@ class RandP(Expr):
         self.kind, self.arg = kind, wrap(arg)
 
 
+class NotAProbabilityVector(ValueError):
+    """A Categorical argument whose rows are not probability vectors (Distributions' ``isprobvec``)."""
+
+
+class Table:
+    """A build-time constant vector or matrix that particle values index (``ws_table``): ``T[s]`` on a vector,
+    ``T[s, k]`` on a matrix, and the row ``T[s, :]`` as the argument of ``Categorical``.  Indices are Julia's,
+    1-based.  An index that is not an integer in range reads NaN and counts an index fault, which :func:`run`
+    reports as ``IndexError`` when the run ends (the reference throws ``BoundsError`` at the statement)."""
+
+    def __init__(self, values):
+        a = np.array(values, dtype=np.float64)
+        if a.ndim not in (1, 2) or a.size == 0:
+            raise ValueError(f"a table is a non-empty vector or matrix (got shape {a.shape})")
+        self.is_vector = a.ndim == 1
+        self.values = np.ascontiguousarray(a[None, :] if self.is_vector else a)
+        self._probvec = None
+
+    @property
+    def shape(self):
+        return self.values.shape
+
+    def __getitem__(self, idx):
+        idx = idx if isinstance(idx, tuple) else (idx,)
+        if self.is_vector:
+            if len(idx) != 1:
+                raise _unsupported("a vector table takes one index")
+            return TableRead(self, 1.0, idx[0])
+        if len(idx) != 2:
+            raise _unsupported("a matrix table takes two indices, `T[s, k]` (or `T[s, :]` as a Categorical argument)")
+        if isinstance(idx[1], slice):
+            if idx[1] != slice(None):
+                raise _unsupported("only a whole row `T[s, :]` can be sliced out of a table")
+            return TableRow(self, idx[0])
+        return TableRead(self, idx[0], idx[1])
+
+    def check_probabilities(self):
+        """every row >= 0 and summing to 1 within sqrt(eps) (Distributions' ``isprobvec``), else NotAProbabilityVector"""
+        if self._probvec is None:
+            v = self.values
+            sums = v.sum(axis=1)
+            bad = np.flatnonzero(~(np.all(v >= 0.0, axis=1) & (np.abs(sums - 1.0) <= math.sqrt(np.finfo(np.float64).eps))))
+            self._probvec = bad.size == 0
+            self._bad_row = int(bad[0]) + 1 if bad.size else 0
+        if not self._probvec:
+            raise NotAProbabilityVector(f"row {self._bad_row} of the Categorical probabilities is not a probability vector "
+                                        f"(entries must be >= 0 and sum to 1): {self.values[self._bad_row - 1]}")
+
+
+def table(values):
+    """``ws.table(array)``: see :class:`Table`."""
+    return values if isinstance(values, Table) else Table(values)
+
+
+class TableRead(Expr):
+    """``T[row, col]`` (1-based, per particle)."""
+
+    def __init__(self, tab, row, col):
+        self.table, self.row, self.col = tab, wrap(row), wrap(col)
+
+
+class TableRow:
+    """``T[row, :]``: a row of a table, the argument of ``Categorical`` (not a value of its own)."""
+
+    def __init__(self, tab, row):
+        self.table, self.row = tab, wrap(row)
+
+
+def _cat_row(p):
+    """The argument of Categorical as a table row: ``T[s, :]`` or a constant probability vector (a one-row table)."""
+    if isinstance(p, TableRow):
+        row = p
+    elif isinstance(p, Expr) and not isinstance(p, Const):
+        raise _unsupported("Categorical with per-particle probability vectors is outside the device-op set (the "
+                           "probabilities must be a constant vector or a row `P[s, :]` of a build-time matrix)")
+    else:
+        v = np.asarray(p.v if isinstance(p, Const) else p, dtype=np.float64)
+        if v.ndim != 1:
+            raise _unsupported("Categorical takes a probability vector")
+        row = TableRow(Table(v), 1.0)
+    row.table.check_probabilities()
+    return row
+
+
+class RandCat(Expr):
+    """A draw of ``Categorical(row)`` inside a sampler expression (one uniform per particle)."""
+
+    def __init__(self, p):
+        self.p = _cat_row(p)
+
+
+class CatLogp(Expr):
+    """``logpdf(Categorical(row), x)``: log p[x] for x in 1..K, -Inf for any other value."""
+
+    def __init__(self, p, x):
+        self.p, self.x = _cat_row(p), wrap(x)
+
+
+def randcat(p): return RandCat(p)
+def cat_logpdf(p, x): return CatLogp(p, x)
+
+
 def randgamma(shape): return RandP("gamma", shape)
 def randpoisson(rate): return RandP("poisson", rate)
 def randn(): return Rand("n")
@@ -219,7 +321,7 @@ def _is_expr(*xs):
 
 
 def _has_draw(e):
-    if isinstance(e, (Rand, RandP)):
+    if isinstance(e, (Rand, RandP, RandCat)):
         return True
     return isinstance(e, Expr) and any(_has_draw(v) for v in vars(e).values() if isinstance(v, (Expr, list, tuple))) or \
         (isinstance(e, (list, tuple)) and any(_has_draw(v) for v in e))
@@ -491,6 +593,21 @@ def lower(e, store):
         if isinstance(a, list):
             raise _unsupported("vector-valued distribution parameters are outside the device-op set")
         return Tokens(a.toks + [({"gamma": L.TOK_RANDGAMMA, "poisson": L.TOK_RANDPOISSON}[e.kind], 0, 0, 0.0)])
+    if isinstance(e, TableRead):
+        r, c = lower(e.row, store), lower(e.col, store)
+        if isinstance(r, list) or isinstance(c, list):
+            raise _unsupported("table indices must be scalar-valued")
+        return Tokens(r.toks + c.toks + [(L.TOK_TABLE, store._table_id(e.table), 0, 0.0)])
+    if isinstance(e, CatLogp):
+        r, x = lower(e.p.row, store), lower(e.x, store)
+        if isinstance(r, list) or isinstance(x, list):
+            raise _unsupported("Categorical values and rows must be scalar-valued")
+        return Tokens(r.toks + x.toks + [(L.TOK_TABLE, store._table_id(e.p.table), 1, 0.0)])
+    if isinstance(e, RandCat):
+        r = lower(e.p.row, store)
+        if isinstance(r, list):
+            raise _unsupported("a Categorical row index must be scalar-valued")
+        return Tokens(r.toks + [(L.TOK_RANDCAT, store._table_id(e.p.table), 0, 0.0)])
     if isinstance(e, Select):
         c, a, b = lower(e.cond, store), lower(e.a, store), lower(e.b, store)
         if isinstance(c, list) or isinstance(a, list) or isinstance(b, list):

@@ -370,9 +370,12 @@ class Parser:
                 self.in_index += 1
                 args, _ = self.parse_args("]")
                 self.in_index -= 1
-                if len(args) != 1:
-                    raise ModelSyntaxError("only a single index `x[e]` is supported (rewrites.jl:170-171)")
-                a = ("index", a, args[0])
+                if len(args) == 2:
+                    a = ("index2", a, args[0], args[1])   # `P[s, k]` / `P[s, :]`: a row or entry of a build-time matrix
+                elif len(args) != 1:
+                    raise ModelSyntaxError("only `x[e]` and `P[i, j]` indices are supported (rewrites.jl:170-171)")
+                else:
+                    a = ("index", a, args[0])
             elif (k, v) == ("op", "{"):
                 self.next()
                 args, _ = self.parse_args("}")
@@ -411,6 +414,8 @@ class Parser:
             return self.parse_atom_paren()
         if (k, v) == ("op", "["):
             return self.parse_bracket()
+        if (k, v) == ("op", ":") and self.in_index > 0 and self.t[self.i] in (("op", ","), ("op", "]")):
+            return ("colon",)   # `P[s, :]`: the whole row
         if (k, v) == ("op", ":"):
             # symbol literal :x
             nm = self.expect("name")[1]
@@ -532,8 +537,10 @@ def _check_expr(ast, pv, fam, stmt):
         raise _unsupported("struct-valued particle columns (`x.p`) are outside the device-op set")
     if tag == "tuple" and _contains_particle(ast, pv):
         raise ModelSyntaxError("Unsupported expression containing a particle variable (tuple)")
-    if tag == "index" and _contains_particle(ast[2], pv):
-        raise _unsupported("particle-dependent indices are outside the device-op set")
+    if tag in ("index", "index2") and any(_contains_particle(i, pv) for i in ast[2:]):
+        # a build-time array indexed by a particle value is a table (expr.Table); a particle variable is not
+        if _contains_particle(ast[1], pv):
+            raise _unsupported("particle-dependent indices into a particle variable are outside the device-op set")
     for x in ast[1:]:
         if isinstance(x, tuple):
             _check_expr(x, pv, fam, stmt)
@@ -800,6 +807,9 @@ def _binop(op, a, b):
     raise ModelSyntaxError(f"unsupported operator {op}")
 
 
+_COLON = object()   # a bare `:` index
+
+
 def ev(ast, env):
     tag = ast[0]
     if tag == "num":
@@ -854,9 +864,21 @@ def ev(ast, env):
         idx = ev(ast[2], ienv)
         if isinstance(base, Expr):
             return Index(base, int(idx) - 1)  # Julia is 1-based
+        if isinstance(idx, Expr) or isinstance(base, expr.Table):
+            return expr.table(base)[idx]      # `mu[s]`: a build-time vector indexed by a particle value
         if isinstance(idx, _Range):
             return np.asarray(base)[[int(i) - 1 for i in idx]]
         return base[int(idx) - 1]
+    if tag == "index2":
+        base, i, j = ev(ast[1], env), ev(ast[2], env), ev(ast[3], env)
+        if isinstance(base, Expr):
+            raise _unsupported("two indices into a particle variable are outside the device-op set")
+        if isinstance(i, Expr) or isinstance(j, Expr):
+            return expr.table(base)[i, slice(None) if j is _COLON else j]
+        a = base.values if isinstance(base, expr.Table) else np.asarray(base)
+        return a[int(i) - 1, :] if j is _COLON else a[int(i) - 1, int(j) - 1]
+    if tag == "colon":
+        return _COLON
     if tag == "field":
         raise _unsupported("property access in a model body is outside the device-op set")
     if tag == "call":
